@@ -49,7 +49,13 @@ def parse():
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE config #3/#4/#5 legs")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run oracle check of the timed state")
     ap.add_argument("--no-streams", dest="streams", action="store_false", help="skip the epsilon-greedy action-stream lines")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (obs, reward, done, winner of a fixed seeded sample of rank 0's envs) "
+                         "as DIR/<name>.npy in float32, about 32 MiB in all, so that two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
 
 
 # ----------------------------------------------------------------------------------------------- clocks
@@ -277,6 +283,24 @@ def traffic_of(key):
         return None, None
 
 
+DUMP_BYTES = 32 << 20
+
+
+def dump_outputs(dirname, obs, reward, done, winner):
+    """The tick's outputs for a fixed seeded sample of envs (the same ids for the same --envs-per-gpu), as float32 .npy files.
+    All values are small integers or bf16 / f32 numbers, so float32 holds them exactly."""
+    import numpy as np
+    import torch
+    n = reward.shape[0]
+    per_env = 4 * (reward[0].numel() + 2 + (obs[0].numel() if obs is not None else 0))
+    k = min(n, DUMP_BYTES // per_env)
+    idx = torch.as_tensor(np.sort(np.random.default_rng(0).choice(n, size=k, replace=False)), device=reward.device)
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in (("obs", obs), ("reward", reward), ("done", done), ("winner", winner)):
+        if t is not None:
+            np.save(os.path.join(dirname, name + ".npy"), t.index_select(0, idx).float().cpu().numpy())
+
+
 def run_ours(a):
     import numpy as np
     import torch
@@ -358,6 +382,8 @@ def run_ours(a):
     assert env_steps == N * a.steps * TPS, (env_steps, N * a.steps * TPS)
     f_reset = (st1["episodes"] - st0["episodes"]) / env_steps
     value = sum_over_ranks(float(env_steps)) / (ms * 1e-3)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, obs, reward, done, winner)
 
     # ---- in-run parity: the timed state itself, on the first and last 2048 env ids of this rank, against the CPU oracle
     parity = None

@@ -8,9 +8,9 @@ player's observation (tron/map.py:67-84), a full grid copy appended to the histo
 Direction enums for the moves (tron/game.py:149-252, tron/player.py:107-132).  Logic is written from the
 normative restatement in SURVEY.md section 8a, not copied.
 
-Pinned by tests/test_py_port.py: same SHA-256 digests as the reference on 2 x 1000 seeded games, and (in the
-authoring container, where /root/reference exists) cell-for-cell equality with the live reference plus a
-printed speed ratio (port 2.4-2.7k env-steps/s/core vs reference 2.5k on the authoring Xeon).
+Pinned by tests/test_py_port.py: same SHA-256 digests as the reference on 2 x 1000 seeded games and cell-for-cell
+equality with the reference's 300 recorded fuzz games.  Measured next to the live reference on one Xeon host, the port
+ran 2.4-2.7k env-steps/s/core against the reference's 2.5k.
 """
 import enum
 import random

@@ -10,7 +10,6 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (authoring container only)")
 
 
 def _has_gpu():
@@ -22,11 +21,8 @@ def _has_gpu():
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir("/root/reference/Deep-Q-learning_TRON")
     have_gpu = None
     for item in items:
-        if "reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present on this box"))
         if "gpu" in item.keywords:
             if have_gpu is None:
                 have_gpu = _has_gpu()

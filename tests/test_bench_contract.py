@@ -50,6 +50,26 @@ def test_our_arm_line():
 
 
 @pytest.mark.gpu
+def test_dump_outputs_follow_the_ticks_played(tmp_path):
+    """--dump-outputs writes the last timed step's outputs; warmup 2 + steps 2 and warmup 1 + steps 3 play the same ticks from the
+    same inputs, so two processes must dump identical arrays while reporting the steps they timed."""
+    import numpy as np
+    small = ["--envs-per-gpu", "65536", "--ticks-per-step", "4", "--no-e2e", "--no-cpu-baseline", "--no-configs", "--no-streams"]
+    runs = {}
+    for steps, warmup in ((2, 2), (3, 1)):
+        out = tmp_path / ("s%d" % steps)
+        d = _run(small + ["--steps", str(steps), "--warmup", str(warmup), "--dump-outputs", str(out)])
+        assert d["steps"] == steps and d["gpu_launches"] == 4 * steps and d["parity_in_run"] is True
+        runs[steps] = {f.stem: np.load(f) for f in sorted(out.glob("*.npy"))}
+        assert sum(f.stat().st_size for f in out.glob("*.npy")) <= 64 << 20
+    a, b = runs[2], runs[3]
+    assert set(a) == {"obs", "reward", "done", "winner"} and a["obs"].shape[1:] == (2, 1, 12, 12) and a["obs"].shape[0] == a["done"].shape[0]
+    for k in a:
+        assert a[k].dtype == np.float32 and np.array_equal(a[k], b[k]), k
+    assert 0 < a["done"].sum() < a["done"].size and set(np.unique(a["winner"])) <= {0.0, 1.0, 2.0}
+
+
+@pytest.mark.gpu
 def test_our_arm_config_legs():
     """the BASELINE config #3 / #4 / #5 legs of the default invocation (small headline so the test stays short)"""
     d = _run(["--steps", "2", "--warmup", "3", "--envs-per-gpu", "65536", "--ticks-per-step", "4", "--no-e2e", "--no-cpu-baseline", "--no-streams"], timeout=900)

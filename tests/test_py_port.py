@@ -1,12 +1,8 @@
-"""The pure-Python loop port (bench.py's reference arm) against the reference's digests and, in the authoring
-container, against the live reference cell for cell."""
+"""The pure-Python loop port (bench.py's reference arm) against fixtures recorded from the reference: digests, pop_up planes,
+slide-mode trajectories and the fuzz games cell for cell."""
 import hashlib
-import os
-import sys
-import time
 
 import numpy as np
-import pytest
 
 from oracle import py_port as pp
 
@@ -60,30 +56,17 @@ def test_port_slide_mode_matches_fixture():
             assert int(done) == int(sl["done"][row]) and (g.winner or 0) == int(sl["winner"][row])
 
 
-@pytest.mark.reference
-def test_port_equals_live_reference_and_costs_the_same():
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-    import make_golden as mg
-    G, U, P = mg.import_reference()
-    rng = np.random.default_rng(3)
-    t_ref = t_port = 0.0
-    steps = 0
-    for _ in range(150):
-        W = int(rng.integers(3, 13))
-        while True:
-            sp = tuple(int(v) for v in rng.integers(0, W, size=4))
-            if sp[:2] != sp[2:]:
-                break
-        ref = mg.new_game(G, P, W, sp)
+def test_port_equals_reference_fuzz_games():
+    """Cell for cell against the reference's own games in fuzz.json (W = H in [3, 16]): per tick, the per-game SHA-256 covers the
+    Tile.value grid, both observations, alive flags, done, winner and both head positions, hashed as make_golden.make_fuzz does."""
+    for g in load_json("fuzz.json"):
+        W, sp = g["W"], g["spawn"]
         port = pp.PyGame(W, W, sp[:2], sp[2:])
-        while not ref.done:
-            a1, a2 = (int(v) for v in rng.integers(0, 4, size=2))
-            t0 = time.perf_counter(); r1, r2, rd = ref.step(a1, a2); t1 = time.perf_counter()
-            p1, p2, pd = port.step(a1, a2); t2 = time.perf_counter()
-            t_ref += t1 - t0; t_port += t2 - t1; steps += 1
-            assert (np.asarray(r1) == np.asarray(p1)).all() and (np.asarray(r2) == np.asarray(p2)).all() and rd == pd
-            assert (ref.winner or 0) == (port.winner or 0)
-            assert [list(p.position) for p in ref.pps] == [list(p) for p in port.pos]
-            assert mg.tiles_of(ref.history[-1].map).tolist() == [[t.value for t in row] for row in port.history[-1].board.cells]
-    print("\n[py_port] %d ticks: reference %.0f steps/s, port %.0f steps/s (ratio %.2f)" % (steps, steps / t_ref, steps / t_port, t_ref / t_port))
-    assert 0.5 < t_ref / t_port < 2.0  # same order of cost as the thing it stands in for
+        h = hashlib.sha256()
+        for a1, a2 in g["actions"]:
+            s1, s2, done = port.step(a1, a2)
+            h.update(np.array([[t.value for t in row] for row in port.history[-1].board.cells], np.int8).tobytes())
+            h.update(s1.astype(np.int8).tobytes()); h.update(s2.astype(np.int8).tobytes())
+            h.update(bytes([int(a) for a in port.alive] + [int(done), port.winner or 0]))
+            h.update(np.array(port.pos, np.int8).tobytes())
+        assert port.done and (port.winner or 0) == g["winner"] and h.hexdigest() == g["sha256"], (W, sp)
