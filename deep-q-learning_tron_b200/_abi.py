@@ -5,7 +5,7 @@ values compiled from the header with gcc.
 """
 import ctypes as C
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 # status
 OK, ERR_INVALID, ERR_UNSUPPORTED, ERR_CUDA, ERR_ALIGN = 0, -1, -2, -3, -4
@@ -69,6 +69,7 @@ class StepArgs(C.Structure):
         ("policy", C.c_int32), ("policy_epsilon", C.c_float),
         ("n_ticks", C.c_int32), ("obs_every_tick", C.c_int32),
         ("obs_terminal", C.c_void_p), ("extra", C.c_void_p),
+        ("obs_prev", C.c_int32), ("pad1", C.c_int32),
     ]
 
 

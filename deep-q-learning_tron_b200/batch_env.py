@@ -6,6 +6,7 @@ ACKTR.py:285-317 auto-reset).  All compute happens in libtron_b200.so through th
 owns the device memory and supplies the stream.
 """
 import ctypes as C
+import weakref
 
 import torch
 
@@ -118,6 +119,7 @@ class BatchedTron:
         self._tmpl = self._tmpl_key = None
         self.counter = 0
         self.counter_dev = None  # device u64; set by use_device_counter() so captured CUDA graphs advance the RNG between replays
+        self._obs_last = None  # (weakref, _version) of the obs tensor that holds the current state's observation (see step)
         nbytes = C.c_size_t()
         _lib.check(self.lib.tron_state_bytes(self.N, self.W, self.H, self.layout, C.byref(nbytes)), "tron_state_bytes")
         with _OnDevice(self.device):
@@ -177,6 +179,21 @@ class BatchedTron:
             setattr(a, k, v)
         return a
 
+    def _obs_written(self, obs):
+        """`obs` now holds the observation of the current state.  Its version is bumped so that a later write by anyone, another
+        env included, is visible as a version change.  Graph capture and the device counter replay state changes without Python
+        seeing them, so nothing is remembered then."""
+        self._obs_last = None
+        if obs.is_inference() or self.counter_dev is not None or torch.cuda.is_current_stream_capturing():
+            return
+        torch.autograd.graph.increment_version(obs)
+        self._obs_last = (weakref.ref(obs), obs._version)
+
+    def _obs_is_prev(self, obs):
+        last = self._obs_last
+        return (last is not None and last[0]() is obs and obs._version == last[1] and self.counter_dev is None
+                and not torch.cuda.is_current_stream_capturing())
+
     def _dev(self, t, dtype, shape=None, name="tensor"):
         """move/cast a user input to a contiguous device tensor and check its shape (the kernels trust sizes)"""
         if t is None:
@@ -210,6 +227,7 @@ class BatchedTron:
         sp = self._dev(spawn, torch.int8, (self.N, 4), "spawn")
         mk = self._dev(mask, torch.uint8, (self.N,), "mask")
         a = self._args(spawn=_ptr(sp), counter=counter, obs_enc=abi.ENC_NONE)
+        self._obs_last = None
         with _OnDevice(self.device):
             _lib.check(self.lib.tron_reset_ex(C.byref(a), _ptr(mk), self._stream()), "tron_reset_ex")
         return self.observe(obs) if self.P else None
@@ -223,6 +241,7 @@ class BatchedTron:
         a = self._args(obs=obs.data_ptr())
         with _OnDevice(self.device):
             _lib.check(self.lib.tron_observe(C.byref(a), self._stream()), "tron_observe")
+        self._obs_written(obs)
         return obs
 
     def step(self, actions=None, spawn=None, slide_tape=None, obs=None, reward=None, done=None, winner=None, ep_len=None,
@@ -230,7 +249,13 @@ class BatchedTron:
         """One tick of every game.  actions: [N,2] uint8/int32/int64 tensor (P1,P2) or None (uniform random policy).
         Output tensors may be passed in to avoid allocation.  obs_terminal: tensor like obs; the rows of games that finished in this
         tick (and were auto-reset) receive the finished game's last frame (DDQN.py:270-308 next_state), other rows are untouched.
-        -> StepResult(obs, reward, done, winner, ep_len)"""
+        -> StepResult(obs, reward, done, winner, ep_len)
+
+        Passing the same `obs` tensor every tick is the fast path: when it is the very tensor this env last wrote (by step,
+        observe or reset), unchanged since by torch's version counter, and the env's state has not changed in between, the
+        kernel is told that the buffer holds the previous observation (tron_step_args.obs_prev) and may store only the parts of
+        each row that this tick changes.  Writes that bypass the version counter (through `.data`, a raw pointer or another
+        library) are not seen: after one, pass the buffer through observe() first, which always writes full rows."""
         counter, cdev, adv = self._take_counter(counter)
         N, dev = self.N, self.device
         if actions is not None:
@@ -250,6 +275,7 @@ class BatchedTron:
         self._out(winner, (N,), torch.uint8, "winner"); self._out(ep_len, (N,), torch.int32, "ep_len")
         if obs_terminal is not None:
             self._out(obs_terminal, (N, 2, self.P, self.W + 2, self.H + 2), _TORCH_OF.get(self.obs_dtype), "obs_terminal")
+        prev = obs is not None and self._obs_is_prev(obs)
         if obs is None and self.P:
             obs = self.new_obs()
         if reward is None:
@@ -262,10 +288,14 @@ class BatchedTron:
             ep_len = torch.empty(N, dtype=torch.int32, device=dev)
         a = self._args(actions=_ptr(actions), action_dtype=0 if actions is None else _CODE_OF[actions.dtype], obs=_ptr(obs),
                        reward=reward.data_ptr(), done=done.data_ptr(), winner=winner.data_ptr(), ep_len_out=_ptr(ep_len),
-                       spawn=_ptr(sp), slide_tape=_ptr(sl), counter=counter, counter_dev=cdev, obs_terminal=_ptr(obs_terminal))
+                       spawn=_ptr(sp), slide_tape=_ptr(sl), counter=counter, counter_dev=cdev, obs_terminal=_ptr(obs_terminal),
+                       obs_prev=int(prev))
+        self._obs_last = None
         with _OnDevice(dev):
             _lib.check(self.lib.tron_step(C.byref(a), self._stream()), "tron_step")
             self._advance(adv)
+        if obs is not None:
+            self._obs_written(obs)
         return StepResult((obs, reward, done, winner, ep_len))
 
     def bind_step(self, actions=None, obs=None, reward=None, done=None, winner=None, ep_len=None, obs_terminal=None):
@@ -293,6 +323,7 @@ class BatchedTron:
         done = torch.empty((T, N), dtype=torch.uint8, device=dev)
         winner = torch.empty((T, N), dtype=torch.uint8, device=dev)
         ep_len = torch.empty((T, N), dtype=torch.int32, device=dev)
+        self._obs_last = None
         a = self._args(actions=_ptr(act), action_dtype=0 if act is None else _CODE_OF[act.dtype], obs=_ptr(obs),
                        reward=reward.data_ptr(), done=done.data_ptr(), winner=winner.data_ptr(), ep_len_out=ep_len.data_ptr(),
                        spawn=_ptr(sp), counter=counter, counter_dev=cdev, n_ticks=T, obs_every_tick=int(obs_every_tick))
@@ -319,6 +350,7 @@ class BatchedTron:
         t = self._dev(tiles, torch.int8, (N, self.W + 2, self.H + 2), "tiles"); h = self._dev(heads, torch.int8, (N, 4), "heads")
         al = self._dev(alive, torch.uint8, (N, 2), "alive"); d = self._dev(done, torch.uint8, (N,), "done")
         w = self._dev(winner, torch.uint8, (N,), "winner"); k = self._dev(ep_len, torch.int32, (N,), "ep_len")
+        self._obs_last = None
         with _OnDevice(self.device):
             _lib.check(self.lib.tron_import_grid(self.state.data_ptr(), self.N, self.W, self.H, self.layout, _ptr(t), _ptr(h),
                                                  _ptr(al), _ptr(d), _ptr(w), _ptr(k), self._stream()), "tron_import_grid")
@@ -382,6 +414,7 @@ class BatchedTron:
     def load_state_dict(self, sd):
         if tuple(sd["geometry"]) != (self.N, self.W, self.H, self.layout):
             raise ValueError("snapshot geometry %s does not match this environment %s" % (tuple(sd["geometry"]), (self.N, self.W, self.H, self.layout)))
+        self._obs_last = None
         self.state.copy_(sd["state"])
         if self.counter_dev is not None:
             self.counter_dev.fill_(int(sd["counter"]))
@@ -428,6 +461,7 @@ class BoundStep:
 
     def __call__(self):
         env = self.env
+        env._obs_last = None
         if not self._dev_counter:
             self._args.counter = env.counter
             env.counter += 1

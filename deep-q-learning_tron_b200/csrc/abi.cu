@@ -126,6 +126,7 @@ int fill_params(const tron_step_args* a, int mode, StepParams& p) {
             if (((uintptr_t)a->obs_terminal & 15u) != 0) return TRON_ERR_ALIGN;
             p.obs_term = a->obs_terminal;
         }
+        p.obs_prev = (p.obs && a->obs_prev) ? 1 : 0;
         p.actions = a->actions; p.action_dtype = a->action_dtype;
         p.reward = a->reward; p.done = a->done; p.winner = a->winner; p.eplen = a->ep_len_out;
         p.slide_tape = a->slide_tape; p.stats = (unsigned long long*)a->stats;
@@ -298,6 +299,7 @@ int tron_step_many(const tron_step_args* args, tron_stream_t stream) {
     if (args->n_ticks < 1) return TRON_ERR_INVALID;
     if (args->obs_terminal && args->n_ticks > 1) return TRON_ERR_UNSUPPORTED;
     p.T = args->n_ticks; p.obs_every_tick = args->obs_every_tick;
+    p.obs_prev = 0;  // tron_step only
     return dispatch(p, MODE_STEP, args->obs_dtype, args->obs_enc, (cudaStream_t)stream);
 }
 

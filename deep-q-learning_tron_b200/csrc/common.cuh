@@ -19,7 +19,8 @@ enum : int {
     DBG_RING_SLOT = 3,    // replay ring slot outside [0, capacity)
     DBG_ENV_OWNER = 4,    // a thread touched an env outside [0, N)
     DBG_HEAD_RANGE = 5,   // head coordinate outside [-1, W] x [-1, H]
-    DBG_BIT_INDEX = 6     // bit-plane index outside [0, 128)
+    DBG_BIT_INDEX = 6,    // bit-plane index outside [0, 128)
+    DBG_OBS_UNIT = 7      // observation delta: unit list slot, game or chunk outside the CTA's rows
 };
 #ifdef TRON_DEBUG
 // one counter pair per translation unit (no relocatable device code needed); each unit registers a reader with the library

@@ -114,6 +114,7 @@ int tron_host_env_create(tron_host_env** out, const tron_step_args* proto, int n
     tron_host_env* e = new (std::nothrow) tron_host_env();
     if (!e) return TRON_ERR_INVALID;
     e->proto = *proto;
+    e->proto.obs_prev = 0;  // device observations are double-buffered: a buffer never holds the previous tick
     if (cudaGetDevice(&e->device) != cudaSuccess) { cudaGetLastError(); delete e; return TRON_ERR_CUDA; }
     e->n_chunks = n_chunks;
     e->planes = planes_of(proto->obs_enc);

@@ -10,7 +10,10 @@
 // is "write zeros".  A thread keeps its game's planes in 64-bit registers: the tick is bit tests/sets, no shared-memory round
 // trip.  For the observation the owning thread expands its planes into an int8 Tile.value tile in shared memory (10x10: one
 // funnel-shift + bit-spread multiply per 4 cells) and the CTA runs the PRMT encode with 16-byte streaming stores.
-// HBM traffic per game-tick: state read + written (32 or 48 B each way) + observation planes + ~28 B metadata.
+// HBM traffic per game-tick: state read + written (32 or 48 B each way) + observation planes + ~28 B metadata.  When the caller
+// says `obs` still holds the previous tick's observation (tron_step_args.obs_prev; BatchedTron.step with the buffer it wrote last),
+// the 10x10 kernels with bf16 / f32 planes store only the 32-byte units whose cells this tick changed: the thread knows them from
+// its pre- and post-tick planes and heads, the CTA scans the per-game counts and encodes just those units (DESIGN §4.1).
 // Measured on B200 (profiles/r2_sweep.jsonl): the LINEAR store schedule below takes the 10x10 kernels from 0.94-0.97 to 0.98 of
 // the measured HBM peak (pop_up 3 planes 0.95 -> 0.98, + const plane 0.94 -> 0.99); a persistent-CTA variant with register
 // prefetch of the next tile was tried and dropped (0.80: it serialises the tick and store phases that otherwise overlap
@@ -158,14 +161,78 @@ __device__ __forceinline__ void expand_tile(const BitCells<SLIDE, W_T>& g, int r
     else expand_tile_generic<SLIDE>(g, r1, c1, r2, c2, dst);
 }
 
+// ------------------------------------------------------------------------------------------------ observation delta
+// tron_step_args.obs_prev: `obs` already holds the observation of every game's pre-tick state, so only the 32-byte units whose
+// cells this tick changes are written.  A unit holds 16 cells (bf16) or 8 (f32) of one plane, so unit boundaries fall on plane
+// boundaries and one unit-in-plane mask per game serves all its lut planes.  int8 planes (144 B) straddle units: full rows.
+constexpr int kDeltaUnit = 32;  // bytes; a full L2 sector, so no partial-sector write reaches HBM
+template <int W_T, int OD, int LP, int MODE>
+struct DeltaObs {
+    static constexpr int ES = OD == TRON_F32 ? 4 : OD == TRON_BF16 ? 2 : 1;
+    static constexpr bool kOn = W_T == 10 && MODE == MODE_STEP && LP > 0 && OD != TRON_I8;
+    static constexpr int CPU = kDeltaUnit / ES;       // cells per unit: 16 (bf16), 8 (f32)
+    static constexpr int UPP = 144 / CPU;             // units per plane: 9, 18
+    static constexpr int CHU = kDeltaUnit / 16;       // 16-byte chunks per unit
+};
+__device__ __forceinline__ int head_cell10(int r, int c) {
+    const int h = (r + 1) * 12 + c + 1;
+    return TRON_DCHECK(h >= 0 && h < 144, DBG_CELL_INDEX) ? h : 0;
+}
+// bit u set: unit u of the lut planes holds an interior cell whose occ or own bit changed (d_lo / d_hi).  The caller adds the
+// cells of heads that moved: a head cell shows the head tile whatever its planes say, and may lie on the border ring.
+template <int CPU>
+__device__ __forceinline__ uint32_t dirty_units10(unsigned long long d_lo, unsigned long long d_hi) {
+    unsigned long long c[3] = {0ull, 0ull, 0ull};  // cell bits of the 12x12 tile
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const unsigned long long d = row_bits10(d_lo, d_hi, r);
+        const int s = (r + 1) * 12 + 1, w = s >> 6, o = s & 63;
+        c[w] |= d << o;
+        if (o + 10 > 64) c[w + 1] |= d >> (64 - o);
+    }
+    uint32_t um = 0;
+#pragma unroll
+    for (int u = 0; u < 144 / CPU; ++u) {
+        const int b = u * CPU;
+        um |= (((c[b >> 6] >> (b & 63)) & ((1ull << CPU) - 1ull)) != 0ull ? 1u : 0u) << u;
+    }
+    return um;
+}
+// CTA-wide exclusive scan of one count per thread (kBitsThreads threads); returns this thread's offset, *total = the sum
+__device__ __forceinline__ int cta_exclusive_scan(int n, int* wsum, int* total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int incl = n;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int v = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+        if (lane >= o) incl += v;
+    }
+    if (lane == 31) wsum[warp] = incl;
+    __syncthreads();
+    int base = 0, sum = 0;
+#pragma unroll
+    for (int w = 0; w < kBitsThreads / 32; ++w) {
+        base += w < warp ? wsum[w] : 0;
+        sum += wsum[w];
+    }
+    *total = sum;
+    return base + incl - n;
+}
+
 // ------------------------------------------------------------------------------------------------ the kernel
-template <bool SLIDE, int W_T, int OD, int LP, bool CP, int CH, int MODE>
+// DELTA: the obs_prev instantiation (single tick, changed units only); every other launch runs DELTA = false, whose code is the
+// full-row kernel unchanged
+template <bool SLIDE, int W_T, int OD, int LP, bool CP, int CH, int MODE, bool DELTA>
 __global__ void __launch_bounds__(kBitsThreads) step_bits_kernel(const StepParams p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int C = W_T ? (W_T + 2) * (W_T + 2) : p.C;
     int8_t* tile = (int8_t*)smem_raw;  // [G][C] Tile.value bytes, only a staging area for the encode
     uint8_t* tflag = (uint8_t*)(tile + ((p.G * C + 15) & ~15));  // [G] "this game just finished" (terminal-frame pass)
     PlaneTab* smtab = (PlaneTab*)(tflag + ((p.G + 15) & ~15));   // [2][3] tables for the linear schedule
+    using DO = DeltaObs<W_T, OD, LP, MODE>;
+    constexpr bool delta = DELTA && DO::kOn;
+    int* wsum = (int*)(smtab + 6);                               // [4] warp sums of the dirty-unit scan
+    uint16_t* dlist = (uint16_t*)(wsum + 4);                     // [<= G * 2P * UPP] game << 8 | unit of the game's row
     const int tid = threadIdx.x;
     // store schedule: linear (one contiguous 512-byte run per warp store) on the 10x10 board; TRON_OPT_ENCODE_VARIANT 8 selects the
     // per-plane schedule of encode_tile() for comparison
@@ -190,6 +257,9 @@ __global__ void __launch_bounds__(kBitsThreads) step_bits_kernel(const StepParam
     const int T = MODE == MODE_STEP ? p.T : 1;
     for (int t = 0; t < T; ++t) {
         bool fin = false;
+        // pre-tick observation inputs (delta path): occ / own words and head cells
+        const unsigned long long occ0_lo = g.occ_lo, occ0_hi = g.occ_hi, own0_lo = g.own_lo, own0_hi = g.own_hi;
+        const int hp1 = delta ? head_cell10(e.r1, e.c1) : 0, hp2 = delta ? head_cell10(e.r2, e.c2) : 0;
         if (MODE != MODE_OBSERVE && owner) {
             BoxRegs bx;
             fin = env_tick<MODE, false, (SLIDE ? FEAT_ALL : FEAT_EPS)>(g, p, e, env, t, tid, bx);  // BITS10 has no slide plane
@@ -213,6 +283,43 @@ __global__ void __launch_bounds__(kBitsThreads) step_bits_kernel(const StepParam
         if constexpr (LP > 0) {
             if (MODE == MODE_OBSERVE || p.obs_every_tick || t == T - 1) {
                 if (owner) expand_tile<SLIDE, W_T, false>(g, e.r1, e.c1, e.r2, e.c2, tile + tid * C);
+                if constexpr (delta) {
+                    {  // T == 1: list the CTA's changed units in row order, then encode and store only those
+                        constexpr int P = Linear144<OD, LP, CP>::P, CPG = Linear144<OD, LP, CP>::CPG;
+                        int n = 0;
+                        uint32_t um = 0;
+                        if (owner) {
+                            const int hn1 = head_cell10(e.r1, e.c1), hn2 = head_cell10(e.r2, e.c2);
+                            um = dirty_units10<DO::CPU>((occ0_lo ^ g.occ_lo) | (own0_lo ^ g.own_lo), (occ0_hi ^ g.occ_hi) | (own0_hi ^ g.own_hi));
+                            if (hn1 != hp1) um |= (1u << (hp1 / DO::CPU)) | (1u << (hn1 / DO::CPU));
+                            if (hn2 != hp2) um |= (1u << (hp2 / DO::CPU)) | (1u << (hn2 / DO::CPU));
+                            n = __popc(um) * 2 * LP;  // the constant plane never changes
+                        }
+                        int total;
+                        int off = cta_exclusive_scan(n, wsum, &total);
+                        if (owner) {
+#pragma unroll
+                            for (int pq = 0; pq < 2 * P; ++pq) {
+                                if (CP && pq % P == LP) continue;
+                                for (uint32_t m = um; m; m &= m - 1u) {
+                                    if (TRON_DCHECK(off < p.G * 2 * LP * DO::UPP, DBG_OBS_UNIT))
+                                        dlist[off] = (uint16_t)((tid << 8) | (pq * DO::UPP + __ffs(m) - 1));
+                                    ++off;
+                                }
+                            }
+                        }
+                        __syncthreads();
+                        uint4* obase = (uint4*)p.obs + (size_t)env0 * CPG;
+                        for (int i = tid; i < total * DO::CHU; i += kBitsThreads) {
+                            const int k = i / DO::CHU;
+                            const uint32_t ent = dlist[k];
+                            const int ge = (int)(ent >> 8), j = (int)(ent & 0xFFu) * DO::CHU + (i - k * DO::CHU);
+                            if (!TRON_DCHECK(ge < nG && j < CPG, DBG_OBS_UNIT)) continue;
+                            st_cs(obase + (size_t)ge * CPG + j, encode_chunk144<OD, LP, CP>(tile, ge, j, p, smtab));
+                        }
+                        continue;  // T == 1: nothing follows in this tick
+                    }
+                }
                 __syncthreads();
                 const int tt = (MODE == MODE_STEP && p.obs_every_tick) ? t : 0;
                 if (linear) encode_tile_linear144<kBitsThreads, OD, LP, CP>(tile, nG, env0, p, tt, smtab);
@@ -235,19 +342,29 @@ static size_t bits_smem(int G, int C, int LP) {
 }
 
 template <bool SLIDE, int W_T, int OD, int LP, bool CP, int CH, int MODE>
-static int launch_bits_one(const StepParams& p, cudaStream_t s) {
+static int launch_bits_one(const StepParams& p_in, cudaStream_t s) {
+    using DO = DeltaObs<W_T, OD, LP, MODE>;
+    StepParams p = p_in;
+    // the delta store covers single ticks of the linear schedule; TRON_OPT_ENCODE_VARIANT 64 forces full rows (A/B timing)
+    if (!DO::kOn || p.T != 1 || (p.variant & (8 | 64))) p.obs_prev = 0;
     const long long n_tiles = ((long long)p.N + p.G - 1) / p.G;
     size_t smem = bits_smem(p.G, p.C, LP);
+    if (p.obs_prev) smem += 4 * sizeof(int) + (size_t)p.G * 2 * LP * DO::UPP * sizeof(uint16_t);
     if (LP > 0 && MODE == MODE_STEP && n_tiles > 8ll * sm_count()) {
         // Cap the resident CTAs per SM by padding the dynamic shared memory: floor(228 KB / (smem + 1 KB reserved)) == cap.  The fused
         // kernels are write streams; with fewer of them per SM than the register limit (8) the DRAM pages see longer bursts
         // (measured: 4 is best for the two-plane kernels, 5 with the slide plane whose tick phase is longer).
         // int8 planes move fewer bytes per CTA: one plane stays uncapped (0.92; 0.78 at 4), three / four planes take 5 (0.985).
-        const long long cap = g_bits_ctas_per_sm > 0 ? g_bits_ctas_per_sm : (OD == TRON_I8 ? (LP == 1 ? 32 : 5) : SLIDE ? 5 : 4);
+        // The delta store writes about a third of the bytes per CTA: 5 (headline 0.361 ms at 4, 0.320 at 5, 0.340 at 6 per tick,
+        // profiles/r3_obs_delta.jsonl).
+        const long long cap = g_bits_ctas_per_sm > 0 ? g_bits_ctas_per_sm : (OD == TRON_I8 ? (LP == 1 ? 32 : 5) : (SLIDE || p.obs_prev) ? 5 : 4);
         const size_t want = (size_t)(228 * 1024) / (size_t)(cap + 1) - 1024 + 256;
         if (want > smem && want <= 200 * 1024) smem = want;
     }
-    auto kern = step_bits_kernel<SLIDE, W_T, OD, LP, CP, CH, MODE>;
+    auto kern = step_bits_kernel<SLIDE, W_T, OD, LP, CP, CH, MODE, false>;
+    if constexpr (DO::kOn) {
+        if (p.obs_prev) kern = step_bits_kernel<SLIDE, W_T, OD, LP, CP, CH, MODE, true>;
+    }
     if (smem > 48 * 1024 && ensure_dynamic_smem((const void*)kern, smem) != TRON_OK) return TRON_ERR_CUDA;
     kern<<<(unsigned)n_tiles, kBitsThreads, smem, s>>>(p);
     return cudaGetLastError() == cudaSuccess ? TRON_OK : TRON_ERR_CUDA;

@@ -132,40 +132,50 @@ __device__ __forceinline__ void encode_tile(const int8_t* tile, int nG, long lon
 // The observation of one game is one contiguous run of 2*P planes; here item j of a game is its j-th 16-byte chunk, whatever
 // plane it falls into, so every warp-wide store is ONE contiguous 512-byte run (encode_tile() instead issues one store per
 // (player, plane) whose lanes follow the cells, i.e. 2*P interleaved runs of 288 B).  Costs a selector recomputation per chunk.
+template <int OD, int LP, bool CP>
+struct Linear144 {
+    static constexpr int C = 144, ES = OD == TRON_F32 ? 4 : OD == TRON_BF16 ? 2 : 1, P = (LP + (CP ? 1 : 0)) > 0 ? LP + (CP ? 1 : 0) : 1;
+    static constexpr int CPC = 16 / ES;           // cells per 16-byte chunk: 8 (bf16), 4 (f32), 16 (i8)
+    static constexpr int CPP = C / CPC;           // chunks per plane: 18, 36, 9
+    static constexpr int CPG = 2 * P * CPP;       // chunks per game
+};
+// chunk j of game e of the tile (both players' planes in row order)
+template <int OD, int LP, bool CP>
+__device__ __forceinline__ uint4 encode_chunk144(const int8_t* tile, int e, int j, const StepParams& p, const PlaneTab* smtab) {
+    using L = Linear144<OD, LP, CP>;
+    const int pq = j / L::CPP, ch = j - pq * L::CPP, pl = pq / L::P, q = pq - pl * L::P;
+    uint32_t o[4];
+    if (CP && q == LP) {
+        uint32_t f[Enc4<OD>::WORDS];
+        Enc4<OD>::fill(p.const_plane, f);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) o[k] = f[k % Enc4<OD>::WORDS];
+    } else {
+        const PlaneTab tb = smtab[pl * 3 + q];
+        const int8_t* cells = tile + e * L::C + ch * L::CPC;
+        if constexpr (L::CPC == 8) {
+            const uint2 w = *(const uint2*)cells;
+            Enc4<OD>::run(tb, cell_selector(w.x), o); Enc4<OD>::run(tb, cell_selector(w.y), o + 2);
+        } else if constexpr (L::CPC == 4) {
+            Enc4<OD>::run(tb, cell_selector(*(const uint32_t*)cells), o);
+        } else {
+            const uint4 w = *(const uint4*)cells;
+            Enc4<OD>::run(tb, cell_selector(w.x), o); Enc4<OD>::run(tb, cell_selector(w.y), o + 1);
+            Enc4<OD>::run(tb, cell_selector(w.z), o + 2); Enc4<OD>::run(tb, cell_selector(w.w), o + 3);
+        }
+    }
+    return make_uint4(o[0], o[1], o[2], o[3]);
+}
 template <int NT, int OD, int LP, bool CP>
 __device__ __forceinline__ void encode_tile_linear144(const int8_t* tile, int nG, long long env0, const StepParams& p, int t, const PlaneTab* smtab,
                                                       void* out = nullptr, const uint8_t* only = nullptr) {
-    constexpr int C = 144, ES = OD == TRON_F32 ? 4 : OD == TRON_BF16 ? 2 : 1, P = (LP + (CP ? 1 : 0)) > 0 ? LP + (CP ? 1 : 0) : 1;
-    constexpr int CPC = 16 / ES;           // cells per 16-byte chunk: 8 (bf16), 4 (f32), 16 (i8)
-    constexpr int CPP = C / CPC;           // chunks per plane: 18, 36, 9
-    constexpr int CPG = 2 * P * CPP;       // chunks per game
+    constexpr int CPG = Linear144<OD, LP, CP>::CPG;
     const size_t tick_off = (size_t)t * (size_t)p.N * CPG * 16;
     uint4* obase = (uint4*)((char*)(out ? out : p.obs) + tick_off) + (size_t)env0 * CPG;
     for (int it = threadIdx.x; it < nG * CPG; it += NT) {
         const int e = it / CPG, j = it - e * CPG;
         if (only && !only[e]) continue;
-        const int pq = j / CPP, ch = j - pq * CPP, pl = pq / P, q = pq - pl * P;
-        uint32_t o[4];
-        if (CP && q == LP) {
-            uint32_t f[Enc4<OD>::WORDS];
-            Enc4<OD>::fill(p.const_plane, f);
-#pragma unroll
-            for (int k = 0; k < 4; ++k) o[k] = f[k % Enc4<OD>::WORDS];
-        } else {
-            const PlaneTab tb = smtab[pl * 3 + q];
-            const int8_t* cells = tile + e * C + ch * CPC;
-            if constexpr (CPC == 8) {
-                const uint2 w = *(const uint2*)cells;
-                Enc4<OD>::run(tb, cell_selector(w.x), o); Enc4<OD>::run(tb, cell_selector(w.y), o + 2);
-            } else if constexpr (CPC == 4) {
-                Enc4<OD>::run(tb, cell_selector(*(const uint32_t*)cells), o);
-            } else {
-                const uint4 w = *(const uint4*)cells;
-                Enc4<OD>::run(tb, cell_selector(w.x), o); Enc4<OD>::run(tb, cell_selector(w.y), o + 1);
-                Enc4<OD>::run(tb, cell_selector(w.z), o + 2); Enc4<OD>::run(tb, cell_selector(w.w), o + 3);
-            }
-        }
-        st_cs(obase + it, make_uint4(o[0], o[1], o[2], o[3]));
+        st_cs(obase + it, encode_chunk144<OD, LP, CP>(tile, e, j, p, smtab));
     }
 }
 

@@ -45,6 +45,7 @@ struct StepParams {
     long long state_off;
     int state_N;
     int variant;          // TRON_OPT_ENCODE_VARIANT
+    int obs_prev;         // tron_step_args.obs_prev, cleared by the launcher when the kernel cannot use it
 };
 
 __device__ __forceinline__ int read_action(const void* actions, int dtype, size_t i) {

@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define TRON_B200_ABI_VERSION 2
+#define TRON_B200_ABI_VERSION 3
 
 typedef void* tron_stream_t; /* cudaStream_t */
 
@@ -214,6 +214,13 @@ typedef struct tron_step_args {
     float* extra;         /* optional device [N,2,2] f32: per player {degree, weight_p} of the game `obs` shows (Game.get_multy,
                              tron/game.py:137-139) taken from slide_params; needs slide_params.  Written by tron_step,
                              tron_step_many (last tick), tron_observe and tron_reset_ex. */
+
+    /* ---- added in ABI version 3 ---- */
+    int32_t obs_prev;     /* tron_step only, a hint: 1 promises that, for every game, `obs` already holds the observation of the game's
+                             state before this call, as the previous call left it, in the same encoding, dtype and lut.  A kernel may
+                             then skip the 32-byte units of a row that this tick does not change (the 10x10 bit-plane layouts with bf16
+                             or f32 observations do); every other kernel writes full rows.  obs_terminal rows are written in full. */
+    int32_t pad1;
 } tron_step_args;
 
 /* ---- library ---- */
@@ -233,7 +240,8 @@ enum {
     TRON_OPT_SPARSE_MIN_CELLS = 1,
     TRON_OPT_TILE_BYTES = 2, /* shared-memory budget of one tile of games in the generic-size fused kernel (default 18432) */
     TRON_OPT_ENCODE_VARIANT = 3, /* experiments (bit mask, 0 = default): 8 = per-plane observation store schedule on 10x10 boards instead of
-                                     the linear one; 32 = element-store observation kernel on the trail layout instead of the bulk-store one */
+                                     the linear one; 32 = element-store observation kernel on the trail layout instead of the bulk-store one;
+                                     64 = full observation rows even when tron_step_args.obs_prev is set */
     TRON_OPT_BITS_CTAS_PER_SM = 4, /* resident CTAs per SM of the fused bit-plane kernels (capped by padding the dynamic shared memory).
                                      0 = default: 4 for the two-plane kernels, 5 with the slide plane -- these kernels are write
                                      streams and FEWER concurrent streams per SM than the register limit of 8 run faster on B200

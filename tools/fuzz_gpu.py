@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Randomised differential test: random (layout, size, encoding, dtype, slide mode, policy, spawn mode, tapes / RNG, step /
-step_many / masked reset / terminal frames / replay ring) configurations, CUDA (through the C ABI) vs the CPU oracle, bit for bit.
+step_many / masked reset / terminal frames / replay ring / one obs buffer reused every tick) configurations, CUDA (through the C ABI) vs the CPU oracle, bit for bit.
 usage: fuzz_gpu.py [seconds] [seed] [--seeds K] [--debug-checks] [--log FILE]
   --seeds K        run K seeds of 60 cases each instead of a time budget
   --debug-checks   (with TRON_B200_DEBUG=1: the range-checked library) print the device-side violation count at the end"""
@@ -68,11 +68,14 @@ def one_case(rng, case):
               env_id_base=int(rng.integers(0, 1 << 20)), slide_mode=slide, slide_rate=float(rng.choice([0.0, 0.15, 0.7])),
               spawn_mode=int(rng.integers(0, 2)), policy=policy, policy_epsilon=float(rng.choice([0.0, 0.05, 0.5])),
               auto_reset=bool(rng.random() < 0.8), reward=str(rng.choice(["ddqn", "survivor", "acktr2"])))
-    desc = "case %d: %s %dx%d N=%d enc=%d dt=%d slide=%d policy=%d auto=%s" % (case, layout, W, H, N, enc, dt, slide, policy, kw["auto_reset"])
-    if os.environ.get("FUZZ_VERBOSE"):
-        print(desc, flush=True)
     g, o = make_pair(N, W, H, **kw)
     a, b = g.reset(), o.reset()
+    # one obs buffer for every plain step (the delta-store path of the 10x10 bit-plane kernels), seeded with full rows by observe()
+    buf = g.env.observe(g.env.new_obs()) if enc != abi.ENC_NONE and rng.random() < 0.5 else None
+    desc = "case %d: %s %dx%d N=%d enc=%d dt=%d slide=%d policy=%d auto=%s reuse_obs=%s" % (case, layout, W, H, N, enc, dt, slide, policy,
+                                                                                         kw["auto_reset"], buf is not None)
+    if os.environ.get("FUZZ_VERBOSE"):
+        print(desc, flush=True)
     assert (a is None and b is None) or np.array_equal(a, b), desc
     if slide == abi.SLIDE_TEMPER:
         assert np.array_equal(g.env.slide_params.cpu().numpy(), o.slide_params), desc + " temper draws"
@@ -98,6 +101,9 @@ def one_case(rng, case):
             res = g.env.step(None if act is None else torch.as_tensor(act), slide_tape=st, obs_terminal=gt)
             assert_same_step(tuple(to_np(x) for x in res), o.step(act, slide_tape=st, obs_terminal=ot), desc + " tick %d" % t)
             assert np.array_equal(to_np(gt), ot), desc + " terminal frames, tick %d" % t
+        elif buf is not None:
+            res = g.env.step(None if act is None else torch.as_tensor(act), slide_tape=st, obs=buf)
+            assert_same_step(tuple(to_np(x) for x in res), o.step(act, slide_tape=st), desc + " tick %d (reused obs)" % t)
         else:
             assert_same_step(g.step(act, slide_tape=st), o.step(act, slide_tape=st), desc + " tick %d" % t)
     if slide == abi.SLIDE_TEMPER:
