@@ -164,14 +164,13 @@ void slice_params(const StepParams& base, int lo, int n, StepParams& p) {
     if (p.eplen) p.eplen = base.eplen + lo;
 }
 
-int dispatch(StepParams& p, int mode, int obs_dtype, int obs_enc, cudaStream_t s) {
+int dispatch(const StepParams& p, int mode, int obs_dtype, int obs_enc, cudaStream_t s) {
     const int kind = mode == MODE_RESET ? 0 : enc_kind_of(obs_enc);
     if (p.layout == TRON_LAYOUT_BITS10) return launch_step_bits10(p, mode, obs_dtype, kind, s);
     if (p.layout == TRON_LAYOUT_BITS) return launch_step_bits(p, mode, obs_dtype, kind, s);
-    if (p.layout == TRON_LAYOUT_TRAIL) return (kind == 0 || mode == MODE_RESET) ? launch_step_trail(p, mode, s) : launch_step_trail_obs(p, mode, obs_dtype, kind, s);
+    if (p.layout == TRON_LAYOUT_TRAIL) return launch_step_trail(p, mode, obs_dtype, kind, s);
     if (mode == MODE_STEP && kind == 0 && p.C >= g_sparse_min_cells) return launch_step_sparse(p, s);
-    if (p.C == 144 && p.Hc == 12) { p.G = tile_envs_c144(p.N); return launch_step_c144(p, mode, obs_dtype, kind, s); }
-    p.G = tile_envs_generic(p.C);
+    if (p.C == 144 && p.Hc == 12) return launch_step_c144(p, mode, obs_dtype, kind, s);
     return launch_step_generic(p, mode, obs_dtype, kind, s);
 }
 

@@ -18,7 +18,7 @@ size_t grid_stride(int layout, int w, int h);
 int fill_params(const tron_step_args* a, int mode, StepParams& p);
 // narrow a whole-batch parameter block to the games [lo, lo+n)
 void slice_params(const StepParams& base, int lo, int n, StepParams& p);
-int dispatch(StepParams& p, int mode, int obs_dtype, int obs_enc, cudaStream_t s);
+int dispatch(const StepParams& p, int mode, int obs_dtype, int obs_enc, cudaStream_t s);
 
 // RAII: run a call on a given device, restore the caller's device afterwards
 struct DeviceGuard {

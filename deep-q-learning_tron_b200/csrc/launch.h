@@ -21,11 +21,11 @@ __host__ __device__ inline int tron_elem(int dt) {
 
 // step_c144.cu (10x10 grids, compile-time geometry) and step_generic.cu (any W,H)
 // enc_kind: 0 none, 1 = 1 lut plane, 2 = 3 lut planes, 3 = 3 lut planes + const plane
+// The fused-kernel launchers choose the games per CTA (p.G) themselves.
 int launch_step_c144(const StepParams& p, int mode, int obs_dtype, int enc_kind, cudaStream_t s);
 int launch_step_generic(const StepParams& p, int mode, int obs_dtype, int enc_kind, cudaStream_t s);
 int launch_step_sparse(const StepParams& p, cudaStream_t s);
-int launch_step_trail(const StepParams& p, int mode, cudaStream_t s);
-int launch_step_trail_obs(const StepParams& p, int mode, int obs_dtype, int enc_kind, cudaStream_t s);
+int launch_step_trail(const StepParams& p, int mode, int obs_dtype, int enc_kind, cudaStream_t s);
 size_t trail_game_bytes_host(int W, int H);
 // export / import take a StepParams with geometry, layout, grid, state_off, state_N and N filled in
 int launch_trail_export(const StepParams& p, int8_t* tiles, int8_t* heads, uint8_t* alive, uint8_t* done, uint8_t* winner, int32_t* ep_len, cudaStream_t s);
@@ -35,9 +35,7 @@ int launch_step_bits10(const StepParams& p, int mode, int obs_dtype, int enc_kin
 int launch_step_bits(const StepParams& p, int mode, int obs_dtype, int enc_kind, cudaStream_t s);
 int launch_bits_export(const StepParams& p, const void* meta, int8_t* tiles, cudaStream_t s);
 int launch_bits_import(const StepParams& p, const int8_t* tiles, bool derive_heads, cudaStream_t s);
-int tile_envs_c144(int n_envs);
 int tile_envs_small_grid(int n_envs);
-int tile_envs_generic(int cells);
 
 int launch_export_meta(const void* meta, int n, int8_t* heads, uint8_t* alive, uint8_t* done, uint8_t* winner, int32_t* ep_len, cudaStream_t s);
 int launch_import_meta(void* meta, int n, int W, int H, const int8_t* heads, const uint8_t* alive, const uint8_t* done, const uint8_t* winner,

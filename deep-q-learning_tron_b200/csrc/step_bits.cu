@@ -18,8 +18,7 @@
 // the measured HBM peak (pop_up 3 planes 0.95 -> 0.98, + const plane 0.94 -> 0.99); a persistent-CTA variant with register
 // prefetch of the next tile was tried and dropped (0.80: it serialises the tick and store phases that otherwise overlap
 // across the CTAs resident on an SM).
-#include "launch.h"
-#include "step_kernels.cuh"
+#include "step_dispatch.cuh"
 
 namespace tron {
 
@@ -351,15 +350,12 @@ static int launch_bits_one(const StepParams& p_in, cudaStream_t s) {
     size_t smem = bits_smem(p.G, p.C, LP);
     if (p.obs_prev) smem += 4 * sizeof(int) + (size_t)p.G * 2 * LP * DO::UPP * sizeof(uint16_t);
     if (LP > 0 && MODE == MODE_STEP && n_tiles > 8ll * sm_count()) {
-        // Cap the resident CTAs per SM by padding the dynamic shared memory: floor(228 KB / (smem + 1 KB reserved)) == cap.  The fused
-        // kernels are write streams; with fewer of them per SM than the register limit (8) the DRAM pages see longer bursts
-        // (measured: 4 is best for the two-plane kernels, 5 with the slide plane whose tick phase is longer).
+        // Resident CTAs per SM, measured: 4 is best for the two-plane kernels, 5 with the slide plane whose tick phase is longer.
         // int8 planes move fewer bytes per CTA: one plane stays uncapped (0.92; 0.78 at 4), three / four planes take 5 (0.985).
         // The delta store writes about a third of the bytes per CTA: 5 (headline 0.361 ms at 4, 0.320 at 5, 0.340 at 6 per tick,
         // profiles/r3_obs_delta.jsonl).
         const long long cap = g_bits_ctas_per_sm > 0 ? g_bits_ctas_per_sm : (OD == TRON_I8 ? (LP == 1 ? 32 : 5) : (SLIDE || p.obs_prev) ? 5 : 4);
-        const size_t want = (size_t)(228 * 1024) / (size_t)(cap + 1) - 1024 + 256;
-        if (want > smem && want <= 200 * 1024) smem = want;
+        smem = smem_for_ctas_per_sm(smem, cap);
     }
     auto kern = step_bits_kernel<SLIDE, W_T, OD, LP, CP, CH, MODE, false>;
     if constexpr (DO::kOn) {
@@ -369,31 +365,12 @@ static int launch_bits_one(const StepParams& p_in, cudaStream_t s) {
     kern<<<(unsigned)n_tiles, kBitsThreads, smem, s>>>(p);
     return cudaGetLastError() == cudaSuccess ? TRON_OK : TRON_ERR_CUDA;
 }
-template <bool SLIDE, int W_T, int OD, int CH, int MODE>
-static int launch_bits_enc(const StepParams& p, int enc_kind, cudaStream_t s) {
-    switch (enc_kind) {
-        case 1: return launch_bits_one<SLIDE, W_T, OD, 1, false, CH, MODE>(p, s);
-        case 2: return launch_bits_one<SLIDE, W_T, OD, 3, false, CH, MODE>(p, s);
-        case 3: return launch_bits_one<SLIDE, W_T, OD, 3, true, CH, MODE>(p, s);
-        default: return TRON_ERR_INVALID;
-    }
-}
-// CH8: cells per encode item of the non-f32 dtypes (8 when C % 8 == 0, else 4 or 1); f32 uses min(CH8, 4) (whole-sector stores)
+// CH8: cells per encode item of the non-f32 dtypes (8 when C % 8 == 0, else 4 or 1)
 template <bool SLIDE, int W_T, int CH8>
 static int launch_bits_geo(const StepParams& p, int mode, int od, int enc_kind, cudaStream_t s) {
-    constexpr int CH32 = CH8 == 8 ? 4 : CH8;
-    if (mode == MODE_RESET) return launch_bits_one<SLIDE, W_T, TRON_I8, 0, false, CH8, MODE_RESET>(p, s);
-    if (mode == MODE_STEP && enc_kind == 0) return launch_bits_one<SLIDE, W_T, TRON_I8, 0, false, CH8, MODE_STEP>(p, s);
-    if (mode == MODE_STEP) {
-        if (od == TRON_BF16) return launch_bits_enc<SLIDE, W_T, TRON_BF16, CH8, MODE_STEP>(p, enc_kind, s);
-        if (od == TRON_F32) return launch_bits_enc<SLIDE, W_T, TRON_F32, CH32, MODE_STEP>(p, enc_kind, s);
-        if (od == TRON_I8) return launch_bits_enc<SLIDE, W_T, TRON_I8, CH8, MODE_STEP>(p, enc_kind, s);
-    } else if (mode == MODE_OBSERVE) {
-        if (od == TRON_BF16) return launch_bits_enc<SLIDE, W_T, TRON_BF16, CH8, MODE_OBSERVE>(p, enc_kind, s);
-        if (od == TRON_F32) return launch_bits_enc<SLIDE, W_T, TRON_F32, CH32, MODE_OBSERVE>(p, enc_kind, s);
-        if (od == TRON_I8) return launch_bits_enc<SLIDE, W_T, TRON_I8, CH8, MODE_OBSERVE>(p, enc_kind, s);
-    }
-    return TRON_ERR_INVALID;
+    return dispatch_obs(mode, od, enc_kind, [&](auto mode_c, auto od_c, auto lp, auto cp) {
+        return launch_bits_one<SLIDE, W_T, od_c, lp, cp, obs_ch(od_c, CH8), mode_c>(p, s);
+    });
 }
 
 int launch_step_bits10(const StepParams& p_in, int mode, int od, int enc_kind, cudaStream_t s) {

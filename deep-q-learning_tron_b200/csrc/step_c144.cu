@@ -11,8 +11,9 @@ int tile_envs_small_grid(int n_envs) {
     g = (g + 15) & ~15;
     return g < 16 ? 16 : (g > 128 ? 128 : g);
 }
-int tile_envs_c144(int n_envs) { return tile_envs_small_grid(n_envs); }
-int launch_step_c144(const StepParams& p, int mode, int obs_dtype, int enc_kind, cudaStream_t s) {
+int launch_step_c144(const StepParams& p_in, int mode, int obs_dtype, int enc_kind, cudaStream_t s) {
+    StepParams p = p_in;
+    p.G = tile_envs_small_grid(p.N);
     return launch_mode<144, 8>(p, mode, obs_dtype, enc_kind, s);
 }
 }  // namespace tron

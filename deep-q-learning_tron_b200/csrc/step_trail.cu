@@ -25,8 +25,7 @@
 // issue active 74 %, DRAM 19 %), so instruction count is what the layout and these tricks buy.
 #include <algorithm>
 
-#include "launch.h"
-#include "step_kernels.cuh"
+#include "step_dispatch.cuh"
 
 namespace tron {
 
@@ -670,36 +669,21 @@ static int launch_trail_obs_one(StepParams p, cudaStream_t s) {
     else step_trail_obs_kernel<OD, LP, CP, 1, MODE><<<grid, kTrailThreads, smem, s>>>(p);
     return cudaGetLastError() == cudaSuccess ? TRON_OK : TRON_ERR_CUDA;
 }
-template <int OD, int MODE>
-static int launch_trail_obs_enc(const StepParams& p, int enc_kind, cudaStream_t s) {
-    switch (enc_kind) {
-        case 1: return launch_trail_obs_one<OD, 1, false, MODE>(p, s);
-        case 2: return launch_trail_obs_one<OD, 3, false, MODE>(p, s);
-        case 3: return launch_trail_obs_one<OD, 3, true, MODE>(p, s);
-        default: return TRON_ERR_INVALID;
-    }
-}
-int launch_step_trail_obs(const StepParams& p, int mode, int od, int enc_kind, cudaStream_t s) {
-    if (mode == MODE_STEP) {
-        if (od == TRON_BF16) return launch_trail_obs_enc<TRON_BF16, MODE_STEP>(p, enc_kind, s);
-        if (od == TRON_F32) return launch_trail_obs_enc<TRON_F32, MODE_STEP>(p, enc_kind, s);
-        if (od == TRON_I8) return launch_trail_obs_enc<TRON_I8, MODE_STEP>(p, enc_kind, s);
-    } else if (mode == MODE_OBSERVE) {
-        if (od == TRON_BF16) return launch_trail_obs_enc<TRON_BF16, MODE_OBSERVE>(p, enc_kind, s);
-        if (od == TRON_F32) return launch_trail_obs_enc<TRON_F32, MODE_OBSERVE>(p, enc_kind, s);
-        if (od == TRON_I8) return launch_trail_obs_enc<TRON_I8, MODE_OBSERVE>(p, enc_kind, s);
-    }
-    return TRON_ERR_INVALID;
-}
-
-int launch_step_trail(const StepParams& p, int mode, cudaStream_t s) {
+// a reset, or a step without observations (MODE_STEP / MODE_RESET only)
+static int launch_trail_tick(const StepParams& p, int mode, cudaStream_t s) {
     const unsigned grid = (unsigned)(((long long)p.N + kTrailThreads - 1) / kTrailThreads);
     const bool lean = p.slide_mode == TRON_SLIDE_NONE && (p.actions != nullptr || p.eps_thr < 0);
     if (mode == MODE_STEP && lean) step_trail_kernel<MODE_STEP, 0><<<grid, kTrailThreads, 0, s>>>(p);
     else if (mode == MODE_STEP) step_trail_kernel<MODE_STEP, FEAT_ALL><<<grid, kTrailThreads, 0, s>>>(p);
-    else if (mode == MODE_RESET) step_trail_kernel<MODE_RESET, 0><<<grid, kTrailThreads, 0, s>>>(p);
-    else return TRON_ERR_UNSUPPORTED;
+    else step_trail_kernel<MODE_RESET, 0><<<grid, kTrailThreads, 0, s>>>(p);
     return cudaGetLastError() == cudaSuccess ? TRON_OK : TRON_ERR_CUDA;
+}
+
+int launch_step_trail(const StepParams& p, int mode, int od, int enc_kind, cudaStream_t s) {
+    return dispatch_obs(mode, od, enc_kind, [&](auto mode_c, auto od_c, auto lp, auto cp) {
+        if constexpr (lp == 0) return launch_trail_tick(p, mode_c, s);
+        else return launch_trail_obs_one<od_c, lp, cp, mode_c>(p, s);
+    });
 }
 
 // ---- export: render Tile.value grids / metadata from the lists; import: rebuild the lists from grids ---------------
