@@ -7,7 +7,7 @@ import os
 import torch
 
 import tron_b200
-from tron_b200.replay import FrameRing, ReplayRing
+from tron_b200.replay import FrameRing, ReplayRing, StateRing
 
 EPSILON_START, ESPILON_END, DECAY_RATE = 1, 0.003, 0.999  # DDQN.py:18-20
 TAU = 0.001             # DDQN.py:21
@@ -226,6 +226,8 @@ def train(n_envs=65536, env_steps=64, device=None, seed=0, obs_dtype=torch.bfloa
 
     replay="frames": the tick kernel writes observations / rewards / done flags straight into a frame-sharing ring (no push);
     replay="ring": explicit (s, a, r, s', d) ring filled by replay_push (round-1 path, kept for comparison).
+    replay="states": a StateRing keeps each tick's env state (42 B per game-tick) and re-simulates the sampled transitions, so the
+    window is ceil(buffer_size / (2 n_envs)) ticks with no slot cap; the env steps one reused observation buffer.
     overlap: launch the gradient all-reduce on a side stream and run the next tick's forward + env step while it is in flight
     (the optimizer step then lands one tick later than in the reference's strictly sequential loop).
     save_every: every that many GAME_CYCLEs write the reference's checkpoint files + a resume bundle into save_dir (DDQN.py:326).
@@ -258,6 +260,9 @@ def train(n_envs=65536, env_steps=64, device=None, seed=0, obs_dtype=torch.bfloa
         n_slots = max(3, min(64, -(-want // rows) + 1))
         frames = FrameRing(env, n_slots, keep_terminal=True, seed=seed)
         obs = frames.begin() if not resume else env.observe(frames.frames_t[0])
+    elif replay == "states":  # buffer_size transitions, at least two ticks
+        frames = StateRing(env, max(2, -(-(buffer_size or MEM_CAPACITY) // rows)), seed=seed)
+        obs = frames.begin(obs=env.new_obs()) if not resume else env.observe()
     else:
         obs = env.reset() if not resume else env.observe()
     events = []
@@ -272,7 +277,7 @@ def train(n_envs=65536, env_steps=64, device=None, seed=0, obs_dtype=torch.bfloa
         ev[1].record()
         if frames is not None:
             env.select_actions(q, epsilon, counter=env.counter, out=frames.actions_slot().view(-1))
-            obs = frames.step().obs
+            obs = (frames.step(obs=obs) if replay == "states" else frames.step()).obs
         else:
             act = env.select_actions(q, epsilon, counter=env.counter)
             term = obs.clone()  # finished games: next_state is their last frame (DDQN.py:270-308), other rows are overwritten below

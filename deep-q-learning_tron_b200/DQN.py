@@ -96,18 +96,20 @@ def learn_step(model, optimizer, batch):
 
 
 def train(model=None, n_envs=4096, iterations=100, learn_steps_per_iter=1, device="cuda", seed=0, log=None, layout="auto", replay="frames",
-          save_every=0, save_dir="save", on_cycle=None, timings=None, amp=False):
+          save_every=0, save_dir="save", on_cycle=None, timings=None, amp=False, buffer_size=None):
     """Batched restatement of DQN.train (DQN.py:135-309): self-play with the survivor reward (step index / 100 / -25 / 0),
     1-plane observations, one smooth-L1 learn step per cycle on a uniform sample, target r or r + gamma * max Q(s').
 
-    replay="frames": the tick kernel fills a frame-sharing ring (no push); "ring": explicit transitions through replay_push.
+    replay="frames": the tick kernel fills a frame-sharing ring (no push); "ring": explicit transitions through replay_push;
+    "states": a StateRing of env states that re-simulates sampled transitions, buffer_size transitions (default: the reference's
+    capacity and at least one cycle of ticks) with no slot cap.
     save_every: write the reference's checkpoint (save/DQN.bak, DQN.py:295) every that many cycles.
     on_cycle(cycle, stats): the numbers the reference logs per cycle (DQN.py:296-306): loss, p1 win rate, mean duration.
     timings: optional dict receiving device times in ms summed over all ticks (q_forward, env_replay, learn).
     amp: run the ACTING forward under bf16 autocast (the learn step stays fp32 like the reference)."""
     import os
     from Net.DQNNet import Net
-    from tron_b200.replay import FrameRing
+    from tron_b200.replay import FrameRing, StateRing
     model = model or Net(in_planes=1, batch_size=BATCH_SIZE, gamma=GAMMA).to(device)
     opt = torch.optim.Adam(model.parameters())
     env = tron_b200.BatchedTron(n_envs, 10, 10, device=device, obs_dtype=torch.float32, obs_enc="lut1", reward="survivor", seed=seed, layout=layout)
@@ -116,6 +118,10 @@ def train(model=None, n_envs=4096, iterations=100, learn_steps_per_iter=1, devic
     if replay == "frames":  # at least the reference's capacity (DQN.py:32) and one cycle of ticks
         frames = FrameRing(env, max(GAME_CYCLE + 1, min(64, -(-MEM_CAPACITY // rows) + 1)), keep_terminal=True, seed=seed)
         obs = frames.begin()
+    elif replay == "states":
+        want = buffer_size or max(MEM_CAPACITY, rows * GAME_CYCLE)
+        frames = StateRing(env, max(2, -(-want // rows)), seed=seed)
+        obs = frames.begin(obs=env.new_obs())
     else:
         mem = ReplayMemory(max(MEM_CAPACITY, rows * GAME_CYCLE), device=device)
         obs = env.reset()
@@ -136,7 +142,7 @@ def train(model=None, n_envs=4096, iterations=100, learn_steps_per_iter=1, devic
             ev[1].record()
             if frames is not None:
                 env.select_actions(q, epsilon, counter=env.counter, out=frames.actions_slot().view(-1))
-                obs = frames.step().obs
+                obs = (frames.step(obs=obs) if replay == "states" else frames.step()).obs
             else:
                 act = env.select_actions(q, epsilon, counter=env.counter)
                 term = obs.clone()

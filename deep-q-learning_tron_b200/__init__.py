@@ -8,7 +8,7 @@ GPU is missing.
 """
 from . import _abi as abi  # noqa: F401
 
-__all__ = ["abi", "lib", "BatchedTron", "ReplayRing"]
+__all__ = ["abi", "lib", "BatchedTron", "ReplayRing", "StateRing"]
 
 
 def __getattr__(name):  # lazy: importing the package must not require torch / a built library
@@ -21,4 +21,7 @@ def __getattr__(name):  # lazy: importing the package must not require torch / a
     if name == "ReplayRing":
         from .replay import ReplayRing
         return ReplayRing
+    if name == "StateRing":
+        from .replay import StateRing
+        return StateRing
     raise AttributeError(name)

@@ -5,7 +5,7 @@ values compiled from the header with gcc.
 """
 import ctypes as C
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 # status
 OK, ERR_INVALID, ERR_UNSUPPORTED, ERR_CUDA, ERR_ALIGN = 0, -1, -2, -3, -4
@@ -91,6 +91,13 @@ class ReplayFrames(C.Structure):
     ]
 
 
+class ReplayStates(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("n_slots", C.c_int32), ("slot_bytes", C.c_int64),
+        ("states", C.c_void_p), ("action", C.c_void_p), ("counter", C.c_void_p), ("slide_params", C.c_void_p),
+    ]
+
+
 def new_step_args(**kw):
     a = StepArgs()
     a.struct_size = C.sizeof(StepArgs)
@@ -151,6 +158,7 @@ EXPORTED_SYMBOLS = (
     "tron_reset", "tron_reset_ex", "tron_step", "tron_observe", "tron_step_many", "tron_export_grid",
     "tron_import_grid", "tron_random_actions", "tron_select_actions", "tron_advance_counter", "tron_minimax_actions", "tron_pop_up",
     "replay_push", "replay_gather", "replay_sample_indices", "replay_sample_gather", "replay_frames_sample_gather",
+    "replay_states_sample_gather",
     "tron_host_env_create", "tron_host_env_destroy", "tron_host_env_reset", "tron_host_env_step",
     "tron_host_env_step_begin", "tron_host_env_step_wait",
     "tron_host_env_state", "tron_host_alloc", "tron_host_free", "tron_host_copy_bandwidth",

@@ -49,6 +49,8 @@ _SIGS = {
     "replay_sample_indices": (C.c_int, [_i64, _i64, _u64, _u64, _vp, _vp]),
     "replay_sample_gather": (C.c_int, [C.POINTER(abi.ReplayRing), _i64, _i64, _u64, _u64, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
     "replay_frames_sample_gather": (C.c_int, [C.POINTER(abi.ReplayFrames), _i64, _i64, _i64, _u64, _u64, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
+    "replay_states_sample_gather": (C.c_int, [C.POINTER(abi.ReplayStates), C.POINTER(abi.StepArgs), _i64, _i64, _i64, _u64, _u64, _vp, _vp, _i,
+                                              _vp, _vp, _vp, _vp, _vp]),
     "tron_host_env_create": (C.c_int, [C.POINTER(_vp), C.POINTER(abi.StepArgs), _i]),
     "tron_host_env_destroy": (C.c_int, [_vp]),
     "tron_host_env_reset": (C.c_int, [_vp, _vp, _vp]),

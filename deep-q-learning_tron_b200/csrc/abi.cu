@@ -423,6 +423,48 @@ int replay_frames_sample_gather(const replay_frames* fr, int64_t first_tick, int
                                               out_done, out_idx, (cudaStream_t)stream);
 }
 
+int replay_states_sample_gather(const replay_states* rs, const tron_step_args* env, int64_t first_tick, int64_t n_ticks, int64_t k, uint64_t seed,
+                                uint64_t counter, void* out_state, void* out_next, int out_dtype, int64_t* out_action, float* out_reward,
+                                float* out_done, int64_t* out_idx, tron_stream_t stream) {
+    if (!rs || rs->struct_size != sizeof(replay_states) || rs->n_slots < 1 || !rs->states || !rs->action) return TRON_ERR_INVALID;
+    if (!env || env->struct_size != sizeof(tron_step_args)) return TRON_ERR_INVALID;
+    if (env->slide_mode == TRON_SLIDE_TAPE) return TRON_ERR_UNSUPPORTED;  // the tape is not recorded (and tron_step's rules would ask for one)
+    tron_step_args a = *env;
+    a.obs = out_state;  // the env's rules for an observation buffer apply to the outputs (non-null, 16-byte aligned)
+    a.obs_terminal = nullptr;
+    StepParams p;
+    const int rc = fill_params(&a, MODE_STEP, p);
+    if (rc != TRON_OK) return rc;
+    if (p.layout != TRON_LAYOUT_BITS10 && p.layout != TRON_LAYOUT_BITS) return TRON_ERR_UNSUPPORTED;
+    if (!p.P) return TRON_ERR_INVALID;
+    if ((p.slide_mode == TRON_SLIDE_ICE || p.slide_mode == TRON_SLIDE_TEMPER) && !rs->counter) return TRON_ERR_INVALID;
+    if (p.slide_mode == TRON_SLIDE_TEMPER && !rs->slide_params) return TRON_ERR_INVALID;
+    const long long meta_off = (long long)((const char*)p.meta - (const char*)p.grid);
+    if (rs->slot_bytes < meta_off + 8ll * p.N || rs->slot_bytes % 16 != 0) return TRON_ERR_INVALID;
+    const long long rows = 2ll * p.N;
+    if (first_tick < 0 || n_ticks <= 0 || n_ticks > rs->n_slots || k <= 0 || k > n_ticks * rows) return TRON_ERR_INVALID;
+    if (!out_state || !out_next || !out_action || !out_reward || !out_done) return TRON_ERR_INVALID;
+    if (out_dtype != TRON_F32 && out_dtype != TRON_BF16) return TRON_ERR_INVALID;
+    if ((((uintptr_t)out_state | (uintptr_t)out_next | (uintptr_t)rs->states) & 15u) != 0) return TRON_ERR_ALIGN;
+    StateSample q;
+    memset(&q, 0, sizeof q);
+    q.states = (const char*)rs->states; q.slot_bytes = rs->slot_bytes; q.meta_off = meta_off;
+    q.action = rs->action; q.counter = (const unsigned long long*)rs->counter;
+    q.slide_params = p.slide_mode == TRON_SLIDE_TEMPER ? rs->slide_params : nullptr;
+    q.first_tick = first_tick; q.n_ticks = n_ticks; q.k = k; q.seed = seed; q.counter_s = counter;
+    q.S = rs->n_slots; q.out_dtype = out_dtype; q.lp = env->obs_enc == TRON_ENC_LUT1 ? 1 : 3; q.env_i8 = env->obs_dtype == TRON_I8;
+    // the constant plane as the env stores it: bf16-rounded, truncated to int8 or exact
+    q.const_val = env->obs_dtype == TRON_BF16 ? __bfloat162float(__float2bfloat16_rn(env->const_plane))
+                : env->obs_dtype == TRON_I8 ? (float)(int8_t)env->const_plane : env->const_plane;
+    q.out_s = out_state; q.out_s2 = out_next; q.out_a = (long long*)out_action; q.out_r = out_reward; q.out_d = out_done;
+    q.out_idx = (long long*)out_idx;
+    // the re-run tick reads the recorded inputs only and writes nothing but its registers
+    p.obs = nullptr; p.actions = nullptr; p.reward = nullptr; p.done = nullptr; p.winner = nullptr; p.eplen = nullptr; p.stats = nullptr;
+    p.spawn = nullptr; p.slide_tape = nullptr; p.extra = nullptr; p.obs_term = nullptr; p.counter_dev = nullptr; p.slide_params = nullptr;
+    p.counter = 0; p.auto_reset = 0; p.obs_prev = 0; p.eps_thr = -1;
+    return launch_replay_states(p, q, (cudaStream_t)stream);
+}
+
 int tron_debug_violations(uint64_t* count, int32_t* first_code) { return debug_violations(count, first_code); }
 
 }  // extern "C"

@@ -195,4 +195,57 @@ __device__ __forceinline__ uint32_t cell_selector(uint32_t w) {
 }
 __device__ __forceinline__ uint32_t lut4(uint32_t t0, uint32_t t1, uint32_t sel) { return __byte_perm(t0, t1, sel); }
 
+// ---------------------------------------------------------------------------------------------
+// uniform sampling WITHOUT replacement as a keyed pseudo-random permutation of [0, size): idx[i] = pi(i).
+// pi = 6-round balanced Feistel network on 2*hb bits (2^(2hb) >= size), round keys from Philox(seed; counter), with
+// cycle-walking (re-apply until the value falls inside [0, size)), which restricts a permutation of the power-of-two domain to a
+// permutation of [0, size).  Every index is independent of the others, so sampling needs no extra launch and no shared state.
+// ---------------------------------------------------------------------------------------------
+struct FeistelPerm {
+    uint32_t key[6];
+    uint32_t mask;
+    int hb;
+    unsigned long long size;
+};
+__device__ __forceinline__ FeistelPerm feistel_make(unsigned long long size, unsigned long long seed, unsigned long long counter) {
+    FeistelPerm f;
+    const uint4 a = philox(seed, counter, 0ull, TAG_SAMPLE, 0), b = philox(seed, counter, 0ull, TAG_SAMPLE, 1);
+    f.key[0] = a.x; f.key[1] = a.y; f.key[2] = a.z; f.key[3] = a.w; f.key[4] = b.x; f.key[5] = b.y;
+    int bits = 1;
+    while (bits < 62 && (1ull << bits) < size) ++bits;
+    f.hb = (bits + 1) >> 1;
+    f.mask = f.hb >= 32 ? 0xFFFFFFFFu : ((1u << f.hb) - 1u);
+    f.size = size;
+    return f;
+}
+__device__ __forceinline__ uint32_t feistel_mix(uint32_t v) {
+    v *= 0x85EBCA6Bu; v ^= v >> 13; v *= 0xC2B2AE35u; v ^= v >> 16;
+    return v;
+}
+__device__ __forceinline__ unsigned long long feistel_apply(const FeistelPerm& f, unsigned long long i) {
+    unsigned long long x = i;
+    do {
+        uint32_t L = (uint32_t)(x >> f.hb) & f.mask, R = (uint32_t)x & f.mask;
+#pragma unroll
+        for (int r = 0; r < 6; ++r) {
+            const uint32_t t = L ^ (feistel_mix(R ^ f.key[r]) & f.mask);
+            L = R; R = t;
+        }
+        x = ((unsigned long long)L << f.hb) | R;
+    } while (x >= f.size);
+    return x;
+}
+
+// what one MODE_STEP tick of env_tick (tick_core.cuh) reports for a game.  A cell accessor that derives from TickOutSink receives
+// it in g.tick_out (the state replay ring re-runs ticks and keeps the result in registers); the others compile without it.
+struct TickOut {
+    float2 reward;
+    uint32_t done, winner;
+};
+struct TickOutSink {
+    TickOut tick_out;
+};
+template <class Cells>
+constexpr bool kTickOutSink = __is_base_of(TickOutSink, Cells);
+
 }  // namespace tron

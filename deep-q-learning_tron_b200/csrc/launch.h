@@ -57,6 +57,23 @@ int launch_replay_sample_gather(const replay_ring* ring, int64_t size, int64_t k
 int launch_replay_frames_sample_gather(const replay_frames* fr, int64_t first_tick, int64_t n_ticks, int64_t k, uint64_t seed, uint64_t counter,
                                        void* out_s, void* out_s2, int out_dtype, int64_t* out_a, float* out_r, float* out_d, int64_t* out_idx,
                                        cudaStream_t st);
+// state replay ring (step_bits.cu): the per-launch inputs besides the env's StepParams (validated by replay_states_sample_gather)
+struct StateSample {
+    const char* states;                   // [S, slot_bytes]
+    long long slot_bytes, meta_off;       // meta_off: the tron_meta array's offset inside a slot
+    const uint8_t* action;                // [S, N, 2]
+    const unsigned long long* counter;    // [S] or NULL
+    const int8_t* slide_params;           // [S, N, 4] or NULL
+    long long first_tick, n_ticks, k;
+    unsigned long long seed, counter_s;   // the sampler's key and counter
+    int S, out_dtype, lp, env_i8;         // lp: lut planes (the const plane, if any, is plane lp); env_i8: the env's tables hold int8
+    float const_val;                      // the const plane as the env's obs dtype stores it
+    void *out_s, *out_s2;
+    long long* out_a;
+    float *out_r, *out_d;
+    long long* out_idx;
+};
+int launch_replay_states(const StepParams& p, const StateSample& q, cudaStream_t s);
 int debug_violations(uint64_t* count, int32_t* first_code);
 
 }  // namespace tron

@@ -438,4 +438,122 @@ int launch_bits_import(const StepParams& p, const int8_t* tiles, bool derive_hea
     return cudaGetLastError() == cudaSuccess ? TRON_OK : TRON_ERR_CUDA;
 }
 
+// ------------------------------------------------------------------------------------------------ state replay ring
+// replay_states_sample_gather: transition u = (tick, row) of the window, drawn by the same Feistel permutation and (tick, row)
+// mapping as replay_frames_sample_gather.  The owning thread loads the game's planes and meta from slot tick % S, re-runs that
+// tick with the recorded actions, counter and game parameters (no auto-reset: the post-tick state IS the terminal frame of a
+// game that finished) and expands the pre- and post-tick states into two Tile.value tiles.  The CTA then encodes the row's
+// player view of both through the env's plane tables, straight into the out dtype.  G transitions per CTA; output row = sample.
+template <bool SLIDE, int W_T>
+__global__ void __launch_bounds__(kBitsThreads) replay_states_kernel(const StepParams p, const StateSample q) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int C = W_T ? (W_T + 2) * (W_T + 2) : p.C;
+    const int CS = (C + 15) & ~15;                         // tile stride
+    PlaneTab* smtab = (PlaneTab*)smem_raw;                 // [2][3] the env's tables as bf16 bit patterns
+    uint8_t* spl = (uint8_t*)(smtab + 6);                  // [G] player of each transition
+    int8_t* tile = (int8_t*)(spl + ((p.G + 15) & ~15));    // [G][2][CS] s, s'
+    const int tid = threadIdx.x;
+    if (tid < 6) {  // int8 envs: widen the table bytes to bf16 (every int8 is exact in bf16), so one encode serves every env dtype
+        PlaneTab t = p.tab[tid / 3][tid % 3];
+        if (q.env_i8) {
+            uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                const int8_t v = (int8_t)(((i < 4 ? t.lo0 : t.lo1) >> (8 * (i & 3))) & 0xFFu);
+                const uint32_t b = (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn((float)v));
+                w[i >> 2] |= (b & 0xFFu) << (8 * (i & 3));
+                w[2 + (i >> 2)] |= (b >> 8) << (8 * (i & 3));
+            }
+            t.lo0 = w[0]; t.lo1 = w[1]; t.hi0 = w[2]; t.hi1 = w[3];
+        }
+        smtab[tid] = t;
+    }
+    const long long row0 = (long long)blockIdx.x * p.G;
+    const int nG = (int)min((long long)p.G, q.k - row0);
+    const long long rows = 2ll * p.N;
+    if (tid < nG) {
+        const long long row = row0 + tid;
+        const unsigned long long u = feistel_apply(feistel_make((unsigned long long)q.n_ticks * (unsigned long long)rows, q.seed, q.counter_s),
+                                                   (unsigned long long)row);
+        const long long tick = q.first_tick + (long long)(u / (unsigned long long)rows), r = (long long)(u % (unsigned long long)rows);
+        const long long slot = tick % q.S, env = r >> 1;
+        const int pl = (int)(r & 1);
+        if (TRON_DCHECK(slot >= 0 && slot < q.S && r >= 0 && r < rows, DBG_RING_SLOT) && TRON_DCHECK(env < p.N, DBG_ENV_OWNER)) {
+            StepParams ps = p;  // this transition's slot: its planes, its counter, its game parameters
+            ps.grid = (int8_t*)(q.states + slot * q.slot_bytes);
+            ps.counter = q.counter ? q.counter[slot] : 0ull;
+            ps.slide_params = q.slide_params ? (int8_t*)q.slide_params + (size_t)slot * p.N * 4 : nullptr;
+            const uint2 m = ((const uint2*)(q.states + slot * q.slot_bytes + q.meta_off))[env];
+            const uchar2 a = ((const uchar2*)(q.action + (size_t)slot * rows))[env];
+            struct Cells : BitCells<SLIDE, W_T>, TickOutSink {} g;  // env_tick leaves reward / done in g.tick_out
+            g.clear(); g.Wr = p.W; g.Hr = p.H;
+            set_planes<SLIDE, W_T>(g, load_planes<SLIDE>(ps, env));
+            EnvState e = unpack_meta(m);
+            int8_t* ts = tile + 2 * tid * CS;
+            expand_tile<SLIDE, W_T, false>(g, e.r1, e.c1, e.r2, e.c2, ts);
+            const int acts[2] = {a.x, a.y};
+            BoxRegs bx;
+            env_tick<MODE_STEP, false, (SLIDE ? FEAT_SLIDE : 0)>(g, ps, e, env, 0, tid, bx, acts);
+            expand_tile<SLIDE, W_T, false>(g, e.r1, e.c1, e.r2, e.c2, ts + CS);
+            q.out_a[row] = (long long)(pl ? a.y : a.x);
+            q.out_r[row] = pl ? g.tick_out.reward.y : g.tick_out.reward.x;
+            q.out_d[row] = (float)g.tick_out.done;
+            if (q.out_idx) q.out_idx[row] = tick * rows + r;
+        }
+        spl[tid] = (uint8_t)pl;
+    }
+    __syncthreads();
+    // encode: frame w (0 = s, 1 = s') of transition gi is P planes of C elements; plane q < lp through table [player][q], plane lp
+    // (popup3_const) the constant
+    const int P = p.P, lp = q.lp, F = P * C;
+    const bool f32 = q.out_dtype == TRON_F32;
+    const int OES = f32 ? 4 : 2;
+    if ((C * OES) % 16 == 0) {  // every plane is whole 16-byte chunks: chunk j of a frame holds 4 (f32) or 8 (bf16) cells of one plane
+        const int CPC = 16 / OES, CPP = C / CPC, CPF = P * CPP;
+        for (int it = tid; it < nG * 2 * CPF; it += kBitsThreads) {
+            const int gw = it / CPF, j = it - gw * CPF, gi = gw >> 1, w = gw & 1;
+            const int pq = j / CPP, ch = j - pq * CPP;
+            if (!TRON_DCHECK(row0 + gi < q.k && pq < P, DBG_OBS_UNIT)) continue;
+            uint32_t o[4];
+            if (pq == lp) {
+                if (f32) Enc4<TRON_F32>::fill(q.const_val, o);
+                else { Enc4<TRON_BF16>::fill(q.const_val, o); o[2] = o[0]; o[3] = o[1]; }
+            } else {
+                const PlaneTab tb = smtab[spl[gi] * 3 + pq];
+                const uint32_t* cells = (const uint32_t*)(tile + gw * CS + ch * CPC);
+                if (f32) Enc4<TRON_F32>::run(tb, cell_selector(cells[0]), o);
+                else { Enc4<TRON_BF16>::run(tb, cell_selector(cells[0]), o); Enc4<TRON_BF16>::run(tb, cell_selector(cells[1]), o + 2); }
+            }
+            uint4* dst = (uint4*)(w ? q.out_s2 : q.out_s) + (size_t)(row0 + gi) * CPF + j;
+            *dst = make_uint4(o[0], o[1], o[2], o[3]);
+        }
+    } else {  // rows that are not whole 16-byte chunks (generic boards): element stores
+        for (int it = tid; it < nG * 2 * F; it += kBitsThreads) {
+            const int gw = it / F, e = it - gw * F, gi = gw >> 1, w = gw & 1;
+            const int pq = e / C, c = e - pq * C;
+            if (!TRON_DCHECK(row0 + gi < q.k && pq < P, DBG_OBS_UNIT)) continue;
+            uint32_t o[4];  // element 0 of a 4-cell encode whose other three selectors are 0
+            const uint32_t sel = (uint32_t)tile[gw * CS + c] & 7u;
+            if (f32) { if (pq == lp) Enc4<TRON_F32>::fill(q.const_val, o); else Enc4<TRON_F32>::run(smtab[spl[gi] * 3 + pq], sel, o); }
+            else { if (pq == lp) Enc4<TRON_BF16>::fill(q.const_val, o); else Enc4<TRON_BF16>::run(smtab[spl[gi] * 3 + pq], sel, o); }
+            const size_t i = (size_t)(row0 + gi) * F + e;
+            if (f32) ((uint32_t*)(w ? q.out_s2 : q.out_s))[i] = o[0];
+            else ((uint16_t*)(w ? q.out_s2 : q.out_s))[i] = (uint16_t)o[0];
+        }
+    }
+}
+
+int launch_replay_states(const StepParams& p_in, const StateSample& q, cudaStream_t s) {
+    StepParams p = p_in;
+    // a few transitions per CTA, about two CTAs per SM once k is large enough
+    const long long two_waves = 2ll * sm_count();
+    p.G = (int)min(32ll, max(1ll, (q.k + two_waves - 1) / two_waves));
+    const size_t smem = 6 * sizeof(PlaneTab) + (size_t)((p.G + 15) & ~15) + (size_t)p.G * 2 * ((p.C + 15) & ~15);
+    const unsigned grid = (unsigned)((q.k + p.G - 1) / p.G);
+    if (p.layout == TRON_LAYOUT_BITS10) replay_states_kernel<false, 10><<<grid, kBitsThreads, smem, s>>>(p, q);
+    else if (p.W == 10 && p.H == 10) replay_states_kernel<true, 10><<<grid, kBitsThreads, smem, s>>>(p, q);
+    else replay_states_kernel<true, 0><<<grid, kBitsThreads, smem, s>>>(p, q);
+    return cudaGetLastError() == cudaSuccess ? TRON_OK : TRON_ERR_CUDA;
+}
+
 }  // namespace tron

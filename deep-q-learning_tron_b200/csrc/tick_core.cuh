@@ -155,8 +155,8 @@ __device__ __forceinline__ int free_neighbours(const Cells& g, const StepParams&
 // One tick of the env whose cells start at `g`.  Updates `e` (fresh game state if it returns true = "rebuild this grid"),
 // writes reward/done/winner/ep_len for (tick t, env) and adds to the striped statistics.  TRACK maintains the dirty boxes.
 // pre_actions: the two actions already fetched (and range-folded by read_action) by a kernel that prefetches its inputs.
-// FEAT: which optional paths are compiled in -- FEAT_SLIDE the ice/temper slide modes, FEAT_EPS the epsilon-greedy proxy policy.  A
-// launcher picks the leanest instantiation the call allows (fewer instructions and registers for the plain tick).
+// Cells deriving from TickOutSink (common.cuh) also receive the tick's reward / done / winner (MODE_STEP); other Cells: no code.
+// FEAT: optional paths compiled in (FEAT_SLIDE ice/temper slides, FEAT_EPS epsilon-greedy proxy); launchers pick the leanest.
 enum : int { FEAT_SLIDE = 1, FEAT_EPS = 2, FEAT_ALL = 3 };
 static_assert(TRON_STAT_EPISODES == 0 && TRON_STAT_P1_WINS == 1 && TRON_STAT_P2_WINS == 2 && TRON_STAT_DRAWS == 3 && TRON_STAT_EP_TICKS == 4 &&
               TRON_STAT_BAD_ACTION == 5 && TRON_STAT_ENV_STEPS == 6, "env_tick's lane-per-field statistics rely on this field order");
@@ -275,7 +275,7 @@ __device__ __forceinline__ bool env_tick(Cells& g, const StepParams& p, EnvState
             e.r1 = r1; e.c1 = c1; e.r2 = r2; e.c2 = c2;
             e.k += 1;
         }
-        if (p.reward) ((float2*)p.reward)[tn] = make_float2(rw0, rw1);
+        if (p.reward) ((float2*)p.reward)[tn] = make_float2(rw0, rw1);  if constexpr (kTickOutSink<Cells>) g.tick_out = TickOut{make_float2(rw0, rw1), done, winner};
         if (p.done) p.done[tn] = (uint8_t)done;
         if (p.winner) p.winner[tn] = (uint8_t)winner;
         if (p.eplen) p.eplen[tn] = fin;

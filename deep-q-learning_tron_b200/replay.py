@@ -1,11 +1,14 @@
 """GPU replay ring behind the reference's replay containers (DQN.py:81-132 ReplayMemory, DDQN.py:167-203 ReplayBuffer).
 
-Two containers:
+Three containers:
   ReplayRing  -- a ring of whole transitions (s, a, r, s', d) in HBM; push and gather are CUDA kernels, uniform sampling without
                  replacement is a keyed permutation evaluated inside the gather (replay_sample_gather: one launch per batch).
   FrameRing   -- the frame-sharing ring of the batched training loops (DDQN.py:264-308, DQN.py:198-252): the tick kernel writes
                  observations / rewards / done flags straight into time slot t % S, next_state of tick t is the frame of tick t+1,
                  so "push" moves no data at all; replay_frames_sample_gather draws a batch in one launch.
+  StateRing   -- the same transitions from the env's bit-plane state: each tick stores the pre-tick state and the actions
+                 (42 B per game-tick on bits10, against 3,467 B for DDQN's frame ring), and replay_states_sample_gather re-runs
+                 the sampled ticks and renders s and s' in one launch, so the horizon can be thousands of ticks.
 """
 import ctypes as C
 
@@ -218,4 +221,111 @@ class FrameRing:
                                                             s2.data_ptr(), _CODE_OF[out_dtype], a.data_ptr(), r.data_ptr(), d.data_ptr(),
                                                             None if idx is None else idx.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream),
                        "replay_frames_sample_gather")
+        return (s, a, r, s2, d, idx) if want_indices else (s, a, r, s2, d)
+
+
+class StateRing:
+    """Replay ring of env states for a BatchedTron on a bit-plane layout: S time slots, each the state blob (planes + meta) BEFORE
+    tick t, the actions of tick t and the RNG counter it ran with (plus the temper mode's game parameters).  A transition
+    (s, a, r, s', d) is re-simulated when it is sampled: the sample kernel re-runs tick t of the game with tron_step's rules and
+    renders the row's view of the pre- and post-tick states, so s' of a finished game is its last frame, as FrameRing's terminal
+    frames.  Drop-in for FrameRing in a training loop:
+
+        ring = StateRing(env, n_slots)
+        obs = ring.begin(obs=buf)                                   # the policy reads `buf`, refreshed in place every tick
+        loop:  env.select_actions(q, eps, counter=env.counter, out=ring.actions_slot().view(-1)); ring.step(obs=buf)
+               batch = ring.sample(64)
+
+    Same (seed, counter) and window as a FrameRing -> the same sampled transitions, bit for bit.  Passing one reused `obs` buffer
+    lets BatchedTron.step store only the parts of each row that a tick changes.
+    """
+
+    def __init__(self, env, n_slots, seed=0):
+        if n_slots < 1:
+            raise ValueError("StateRing needs at least 1 slot")
+        if env.layout not in (abi.LAYOUT_BITS10, abi.LAYOUT_BITS):
+            raise ValueError("StateRing re-runs ticks on bit-plane states: the env needs layout 'bits10' or 'bits' (got layout %d)" % env.layout)
+        if env.slide_mode == abi.SLIDE_TAPE:
+            raise ValueError("StateRing cannot replay slide_mode='tape': the tape is not recorded")
+        if not env.P:
+            raise ValueError("StateRing needs an environment with observations (obs_enc != 'none')")
+        if not env.auto_reset:
+            raise ValueError("StateRing needs auto_reset=True: a frozen finished game has no next state")
+        self.lib = _lib.load()
+        self.env, self.device = env, env.device
+        self.S, self.rows = int(n_slots), 2 * env.N
+        self.frame_shape = (env.P, env.W + 2, env.H + 2)
+        N = env.N
+        meta_off = C.c_size_t()
+        _lib.check(self.lib.tron_state_offsets(N, env.W, env.H, env.layout, None, C.byref(meta_off), None), "tron_state_offsets")
+        self.state_bytes = meta_off.value + 8 * N  # planes + meta: what a tick reads (the dirty boxes are the sparse kernel's)
+        slot_bytes = (self.state_bytes + 15) & ~15
+        self.states_t = torch.zeros((self.S, slot_bytes), dtype=torch.uint8, device=self.device)
+        self.action_t = torch.zeros((self.S, N, 2), dtype=torch.uint8, device=self.device)
+        self.counter_t = torch.zeros(self.S, dtype=torch.int64, device=self.device)
+        self.params_t = torch.zeros((self.S, N, 4), dtype=torch.int8, device=self.device) if env.slide_mode == abi.SLIDE_TEMPER else None
+        self.tick = 0  # ticks played: transitions of ticks [max(0, tick - S), tick) are in the ring
+        self.seed, self.sample_counter = int(seed), 0
+        self.rs = abi.ReplayStates(struct_size=C.sizeof(abi.ReplayStates), n_slots=self.S, slot_bytes=slot_bytes, states=self.states_t.data_ptr(),
+                                   action=self.action_t.data_ptr(), counter=self.counter_t.data_ptr(),
+                                   slide_params=None if self.params_t is None else self.params_t.data_ptr())
+
+    def __len__(self):
+        return min(self.tick, self.S) * self.rows
+
+    def begin(self, spawn=None, obs=None):
+        """reset the env (its first observation lands in `obs`, default a new buffer) and start at tick 0"""
+        self.tick = 0
+        return self.env.reset(spawn=spawn, obs=obs)
+
+    def actions_slot(self):
+        """uint8 [N,2] view the policy writes the actions of the current tick into (select_actions(out=...))"""
+        return self.action_t[self.tick % self.S]
+
+    def step(self, actions=None, obs=None, **kw):
+        """record the pre-tick state, then one env tick; actions None -> the ones already written into actions_slot().
+        All on the env's stream, so the step can be captured in a CUDA graph (with env.use_device_counter())."""
+        env, slot = self.env, self.tick % self.S
+        if actions is not None:
+            self.action_t[slot].copy_(actions.reshape(env.N, 2))
+        self.states_t[slot, :self.state_bytes].copy_(env.state[:self.state_bytes])
+        if kw.get("counter") is not None:
+            self.counter_t[slot].fill_(int(kw["counter"]))
+        elif env.counter_dev is not None:
+            self.counter_t[slot:slot + 1].copy_(env.counter_dev)
+        else:
+            self.counter_t[slot].fill_(env.counter)
+        if self.params_t is not None:
+            self.params_t[slot].copy_(env.slide_params)
+        res = env.step(self.action_t[slot], obs=obs, want_ep_len=False, **kw)
+        self.tick += 1
+        return res
+
+    def sample(self, k, out_dtype=torch.float32, counter=None, want_indices=False, out=None):
+        """k distinct transitions of the last min(tick, S) ticks, uniformly, one launch -> (s, a i64 [k,1], r f32 [k,1], s', d f32 [k,1]),
+        as FrameRing.sample.  out: the 5-tuple a previous call returned, to write into the same tensors again."""
+        n_ticks = min(self.tick, self.S)
+        if counter is None:
+            counter, self.sample_counter = self.sample_counter, self.sample_counter + 1
+        if not 0 < k <= n_ticks * self.rows:
+            raise ValueError("sample: need 0 < k <= %d transitions, got %d" % (n_ticks * self.rows, k))
+        if out_dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError("out_dtype must be float32 or bfloat16")
+        if out is not None:
+            s, a, r, s2, d = out[:5]
+            if s.shape[0] != k or s.dtype != out_dtype or tuple(s.shape[1:]) != self.frame_shape:
+                raise ValueError("sample: `out` does not match k / out_dtype / the frame shape")
+        else:
+            s = torch.empty((k,) + self.frame_shape, dtype=out_dtype, device=self.device)
+            s2 = torch.empty_like(s)
+            a = torch.empty((k, 1), dtype=torch.int64, device=self.device)
+            r = torch.empty((k, 1), dtype=torch.float32, device=self.device)
+            d = torch.empty((k, 1), dtype=torch.float32, device=self.device)
+        idx = torch.empty(k, dtype=torch.int64, device=self.device) if want_indices else None
+        args = self.env._args()
+        with _OnDevice(self.device):
+            _lib.check(self.lib.replay_states_sample_gather(C.byref(self.rs), C.byref(args), self.tick - n_ticks, n_ticks, k, self.seed, counter,
+                                                            s.data_ptr(), s2.data_ptr(), _CODE_OF[out_dtype], a.data_ptr(), r.data_ptr(), d.data_ptr(),
+                                                            None if idx is None else idx.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream),
+                       "replay_states_sample_gather")
         return (s, a, r, s2, d, idx) if want_indices else (s, a, r, s2, d)

@@ -19,6 +19,8 @@
  *   DDQN.py:167-203        ReplayBuffer             -> replay_push / replay_gather / replay_sample_indices / replay_sample_gather
  *   DDQN.py:264-308, DQN.py:198-252   per-transition replay fill of the training loops -> replay_frames (the tick kernel writes
  *                          observations, rewards and done flags straight into the ring; replay_frames_sample_gather reads them back)
+ *                          or replay_states (the ring keeps each tick's env state and actions; replay_states_sample_gather re-runs
+ *                          the sampled ticks and renders both frames)
  *
  * Conventions
  *   - Every entry point is extern "C", returns 0 (TRON_OK) or a negative tron_status, never throws.
@@ -43,7 +45,7 @@
 extern "C" {
 #endif
 
-#define TRON_B200_ABI_VERSION 3
+#define TRON_B200_ABI_VERSION 4
 
 typedef void* tron_stream_t; /* cudaStream_t */
 
@@ -376,6 +378,33 @@ typedef struct replay_frames {
  * tick * rows + row of each sample. */
 int replay_frames_sample_gather(const replay_frames* fr, int64_t first_tick, int64_t n_ticks, int64_t k, uint64_t seed,
                                 uint64_t counter, void* out_state, void* out_next, int out_dtype, int64_t* out_action,
+                                float* out_reward, float* out_done, int64_t* out_idx, tron_stream_t stream);
+
+/* ---- state replay ring (ABI 4): the same transitions from 42 bytes per game-tick (TRON_LAYOUT_BITS10) ----
+ * Slot (t % S) holds the env's state blob BEFORE tick t (its first slot_bytes bytes: the bit planes and the tron_meta array, i.e.
+ * meta_off + 8*N of tron_state_offsets, rounded up to 16), the two actions of tick t and, when the tick draws slide numbers, the
+ * RNG counter it ran with and the temper mode's per-game parameters.  A transition (s, a, r, s', d) is a function of those: the
+ * sampler re-runs the tick (tron_step's rules, no auto-reset), so s' of a game that finished is its last frame, as with
+ * replay_frames.terminal.  Bit-plane layouts only (TRON_LAYOUT_BITS10, TRON_LAYOUT_BITS), every slide mode but TRON_SLIDE_TAPE. */
+typedef struct replay_states {
+    uint32_t struct_size;
+    int32_t n_slots;        /* S >= 1 */
+    int64_t slot_bytes;     /* >= meta_off + 8*N, a multiple of 16 */
+    void* states;           /* device [S, slot_bytes], 16-byte aligned */
+    uint8_t* action;        /* device [S, N, 2] */
+    uint64_t* counter;      /* device [S]: the counter tick t ran with (tron_step_args.counter + *counter_dev); needed for ICE / TEMPER */
+    int8_t* slide_params;   /* device [S, N, 4]: {degree, weight1, weight2, 0} of each game during tick t; needed for TEMPER */
+} replay_states;
+/* Sample k distinct transitions uniformly among ticks [first_tick, first_tick + n_ticks) x 2N rows (n_ticks <= S: s' is
+ * recomputed, no slot holds it) and render them, one launch.  The same (seed, counter) picks the same (tick, row) as
+ * replay_frames_sample_gather over the same window.  `env` is the argument block of the env the ring records: it supplies the
+ * geometry, layout, encoding, obs dtype, lut, const plane, reward table, slide mode and rate, seed and env_id_base, and is
+ * validated like a tron_step call (its obs, actions and output pointers are not used; its state pointer is not read).  Every output
+ * element is what tron_step would have stored in the env's obs dtype, converted to out_dtype (TRON_F32 | TRON_BF16) as
+ * replay_frames_sample_gather converts; outputs, alignment and out_idx (tick * 2N + row) as there.  TRON_ERR_UNSUPPORTED for
+ * the other layouts and for TRON_SLIDE_TAPE. */
+int replay_states_sample_gather(const replay_states* rs, const tron_step_args* env, int64_t first_tick, int64_t n_ticks, int64_t k,
+                                uint64_t seed, uint64_t counter, void* out_state, void* out_next, int out_dtype, int64_t* out_action,
                                 float* out_reward, float* out_done, int64_t* out_idx, tron_stream_t stream);
 
 /* ---- host-buffer front end (what a Game.step caller with numpy arrays binds to) ---- */
