@@ -254,15 +254,14 @@ def train(n_envs=65536, env_steps=64, device=None, seed=0, obs_dtype=torch.bfloa
         extra = agent.load(resume, env)
         epsilon = float(extra.get("epsilon", epsilon)); start_tick = int(extra.get("tick", 0))
     rows = 2 * n_envs
-    frames = None
+    want = buffer_size or MEM_CAPACITY
+    ring = None
     if replay == "frames":
-        want = buffer_size or MEM_CAPACITY
-        n_slots = max(3, min(64, -(-want // rows) + 1))
-        frames = FrameRing(env, n_slots, keep_terminal=True, seed=seed)
-        obs = frames.begin() if not resume else env.observe(frames.frames_t[0])
+        ring = FrameRing(env, max(3, min(64, -(-want // rows) + 1)), keep_terminal=True, seed=seed)
     elif replay == "states":  # buffer_size transitions, at least two ticks
-        frames = StateRing(env, max(2, -(-(buffer_size or MEM_CAPACITY) // rows)), seed=seed)
-        obs = frames.begin(obs=env.new_obs()) if not resume else env.observe()
+        ring = StateRing(env, max(2, -(-want // rows)), seed=seed)
+    if ring is not None:
+        obs = ring.begin() if not resume else env.observe(ring.obs)
     else:
         obs = env.reset() if not resume else env.observe()
     events = []
@@ -275,9 +274,9 @@ def train(n_envs=65536, env_steps=64, device=None, seed=0, obs_dtype=torch.bfloa
         ev[0].record()
         q = agent.q_values(obs.view(rows, 3, 12, 12), amp=amp)
         ev[1].record()
-        if frames is not None:
-            env.select_actions(q, epsilon, counter=env.counter, out=frames.actions_slot().view(-1))
-            obs = (frames.step(obs=obs) if replay == "states" else frames.step()).obs
+        if ring is not None:
+            env.select_actions(q, epsilon, counter=env.counter, out=ring.actions_slot().view(-1))
+            obs = ring.step().obs
         else:
             act = env.select_actions(q, epsilon, counter=env.counter)
             term = obs.clone()  # finished games: next_state is their last frame (DDQN.py:270-308), other rows are overwritten below
@@ -287,10 +286,10 @@ def train(n_envs=65536, env_steps=64, device=None, seed=0, obs_dtype=torch.bfloa
             obs = res.obs
         ev[2].record()
         agent.learn_finish()  # the learn step begun last tick: its all-reduce ran behind this tick's forward + env step
-        have = len(frames) if frames is not None else len(agent.memory)
+        have = len(ring) if ring is not None else len(agent.memory)
         if (t + 1) % learn_every == 0 and have > batch:
             # the sampled batch is consumed by backward before the next learn step, so its buffers are reused
-            exp = sample_bufs = (frames.sample(batch, out=sample_bufs) if frames is not None else agent.memory.sample())
+            exp = sample_bufs = (ring.sample(batch, out=sample_bufs) if ring is not None else agent.memory.sample())
             n_learn += 1
             if overlap:
                 agent.learn_begin(exp)

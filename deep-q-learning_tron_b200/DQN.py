@@ -114,17 +114,15 @@ def train(model=None, n_envs=4096, iterations=100, learn_steps_per_iter=1, devic
     opt = torch.optim.Adam(model.parameters())
     env = tron_b200.BatchedTron(n_envs, 10, 10, device=device, obs_dtype=torch.float32, obs_enc="lut1", reward="survivor", seed=seed, layout=layout)
     rows = 2 * n_envs
-    frames = mem = None
+    ring = mem = None
     if replay == "frames":  # at least the reference's capacity (DQN.py:32) and one cycle of ticks
-        frames = FrameRing(env, max(GAME_CYCLE + 1, min(64, -(-MEM_CAPACITY // rows) + 1)), keep_terminal=True, seed=seed)
-        obs = frames.begin()
+        ring = FrameRing(env, max(GAME_CYCLE + 1, min(64, -(-MEM_CAPACITY // rows) + 1)), keep_terminal=True, seed=seed)
     elif replay == "states":
         want = buffer_size or max(MEM_CAPACITY, rows * GAME_CYCLE)
-        frames = StateRing(env, max(2, -(-want // rows)), seed=seed)
-        obs = frames.begin(obs=env.new_obs())
+        ring = StateRing(env, max(2, -(-want // rows)), seed=seed)
     else:
         mem = ReplayMemory(max(MEM_CAPACITY, rows * GAME_CYCLE), device=device)
-        obs = env.reset()
+    obs = ring.begin() if ring is not None else env.reset()
     epsilon = float(EPSILON_START)
     losses = []
     events, learn_events = [], []
@@ -140,9 +138,9 @@ def train(model=None, n_envs=4096, iterations=100, learn_steps_per_iter=1, devic
                 else:
                     q = model(obs.view(rows, 1, 12, 12))
             ev[1].record()
-            if frames is not None:
-                env.select_actions(q, epsilon, counter=env.counter, out=frames.actions_slot().view(-1))
-                obs = (frames.step(obs=obs) if replay == "states" else frames.step()).obs
+            if ring is not None:
+                env.select_actions(q, epsilon, counter=env.counter, out=ring.actions_slot().view(-1))
+                obs = ring.step().obs
             else:
                 act = env.select_actions(q, epsilon, counter=env.counter)
                 term = obs.clone()
@@ -157,9 +155,9 @@ def train(model=None, n_envs=4096, iterations=100, learn_steps_per_iter=1, devic
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(learn_steps_per_iter):
-            have = len(frames) if frames is not None else len(mem)
+            have = len(ring) if ring is not None else len(mem)
             k = min(have, model.batch_size)
-            batch = frames.sample(k) if frames is not None else mem.sample_batch(k)
+            batch = ring.sample(k) if ring is not None else mem.sample_batch(k)
             losses.append(learn_step(model, opt, batch))
         e1.record()
         learn_events.append((e0, e1))

@@ -380,6 +380,14 @@ static int ring_ok(const replay_ring* r) {
     return r->state && r->next_state && r->action && r->reward && r->done;
 }
 
+// the outputs of the sample / gather entry points: five buffers, f32 or bf16 frames, 16-byte aligned like the ring's (NULL passes)
+static int check_batch_outputs(const void* out_state, const void* out_next, int out_dtype, const void* out_action, const void* out_reward,
+                               const void* out_done, const void* ring_a, const void* ring_b) {
+    if (!out_state || !out_next || !out_action || !out_reward || !out_done) return TRON_ERR_INVALID;
+    if (out_dtype != TRON_F32 && out_dtype != TRON_BF16) return TRON_ERR_INVALID;
+    return (((uintptr_t)out_state | (uintptr_t)out_next | (uintptr_t)ring_a | (uintptr_t)ring_b) & 15u) != 0 ? TRON_ERR_ALIGN : TRON_OK;
+}
+
 int replay_push(const replay_ring* ring, uint64_t cursor, const void* state, const void* next_state, const uint8_t* action,
                 const float* reward, const uint8_t* done, int done_stride, int64_t n, tron_stream_t stream) {
     if (!ring_ok(ring) || !state || !next_state || !action || !reward || !done) return TRON_ERR_INVALID;
@@ -389,9 +397,8 @@ int replay_push(const replay_ring* ring, uint64_t cursor, const void* state, con
 
 int replay_gather(const replay_ring* ring, const int64_t* idx, int64_t k, void* out_state, void* out_next, int out_dtype,
                   int64_t* out_action, float* out_reward, float* out_done, tron_stream_t stream) {
-    if (!ring_ok(ring) || !idx || k <= 0 || !out_state || !out_next || !out_action || !out_reward || !out_done) return TRON_ERR_INVALID;
-    if (out_dtype != TRON_F32 && out_dtype != TRON_BF16) return TRON_ERR_INVALID;
-    if ((((uintptr_t)out_state | (uintptr_t)out_next | (uintptr_t)ring->state | (uintptr_t)ring->next_state) & 15u) != 0) return TRON_ERR_ALIGN;
+    if (!ring_ok(ring) || !idx || k <= 0) return TRON_ERR_INVALID;
+    if (const int rc = check_batch_outputs(out_state, out_next, out_dtype, out_action, out_reward, out_done, ring->state, ring->next_state)) return rc;
     return launch_replay_gather(ring, idx, k, out_state, out_next, out_dtype, out_action, out_reward, out_done, (cudaStream_t)stream);
 }
 
@@ -402,9 +409,8 @@ int replay_sample_indices(int64_t size, int64_t k, uint64_t seed, uint64_t count
 
 int replay_sample_gather(const replay_ring* ring, int64_t size, int64_t k, uint64_t seed, uint64_t counter, void* out_state, void* out_next,
                          int out_dtype, int64_t* out_action, float* out_reward, float* out_done, int64_t* out_idx, tron_stream_t stream) {
-    if (!ring_ok(ring) || k <= 0 || k > size || size > ring->capacity || !out_state || !out_next || !out_action || !out_reward || !out_done) return TRON_ERR_INVALID;
-    if (out_dtype != TRON_F32 && out_dtype != TRON_BF16) return TRON_ERR_INVALID;
-    if ((((uintptr_t)out_state | (uintptr_t)out_next | (uintptr_t)ring->state | (uintptr_t)ring->next_state) & 15u) != 0) return TRON_ERR_ALIGN;
+    if (!ring_ok(ring) || k <= 0 || k > size || size > ring->capacity) return TRON_ERR_INVALID;
+    if (const int rc = check_batch_outputs(out_state, out_next, out_dtype, out_action, out_reward, out_done, ring->state, ring->next_state)) return rc;
     return launch_replay_sample_gather(ring, size, k, seed, counter, out_state, out_next, out_dtype, out_action, out_reward, out_done, out_idx,
                                        (cudaStream_t)stream);
 }
@@ -416,9 +422,7 @@ int replay_frames_sample_gather(const replay_frames* fr, int64_t first_tick, int
     if (fr->frame_dtype != TRON_BF16 && fr->frame_dtype != TRON_F32 && fr->frame_dtype != TRON_I8) return TRON_ERR_INVALID;
     if (!fr->frames || !fr->action || !fr->reward || !fr->done) return TRON_ERR_INVALID;
     if (first_tick < 0 || n_ticks <= 0 || n_ticks > fr->n_slots - 1 || k <= 0 || k > n_ticks * fr->rows) return TRON_ERR_INVALID;
-    if (!out_state || !out_next || !out_action || !out_reward || !out_done) return TRON_ERR_INVALID;
-    if (out_dtype != TRON_F32 && out_dtype != TRON_BF16) return TRON_ERR_INVALID;
-    if ((((uintptr_t)out_state | (uintptr_t)out_next | (uintptr_t)fr->frames | (uintptr_t)fr->terminal) & 15u) != 0) return TRON_ERR_ALIGN;
+    if (const int rc = check_batch_outputs(out_state, out_next, out_dtype, out_action, out_reward, out_done, fr->frames, fr->terminal)) return rc;
     return launch_replay_frames_sample_gather(fr, first_tick, n_ticks, k, seed, counter, out_state, out_next, out_dtype, out_action, out_reward,
                                               out_done, out_idx, (cudaStream_t)stream);
 }
@@ -443,9 +447,7 @@ int replay_states_sample_gather(const replay_states* rs, const tron_step_args* e
     if (rs->slot_bytes < meta_off + 8ll * p.N || rs->slot_bytes % 16 != 0) return TRON_ERR_INVALID;
     const long long rows = 2ll * p.N;
     if (first_tick < 0 || n_ticks <= 0 || n_ticks > rs->n_slots || k <= 0 || k > n_ticks * rows) return TRON_ERR_INVALID;
-    if (!out_state || !out_next || !out_action || !out_reward || !out_done) return TRON_ERR_INVALID;
-    if (out_dtype != TRON_F32 && out_dtype != TRON_BF16) return TRON_ERR_INVALID;
-    if ((((uintptr_t)out_state | (uintptr_t)out_next | (uintptr_t)rs->states) & 15u) != 0) return TRON_ERR_ALIGN;
+    if (const int out_rc = check_batch_outputs(out_state, out_next, out_dtype, out_action, out_reward, out_done, rs->states, nullptr)) return out_rc;
     StateSample q;
     memset(&q, 0, sizeof q);
     q.states = (const char*)rs->states; q.slot_bytes = rs->slot_bytes; q.meta_off = meta_off;

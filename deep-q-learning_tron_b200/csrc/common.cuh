@@ -248,4 +248,14 @@ struct TickOutSink {
 template <class Cells>
 constexpr bool kTickOutSink = __is_base_of(TickOutSink, Cells);
 
+// the transition that sample `row` of a window replay ring draws: u = pi(row) over the window's n_ticks * rows transitions, then
+// (tick, r) = (first_tick + u / rows, u % rows).  The frame ring and the state ring both sample through this one mapping, which is
+// what makes them hand out the same transitions for the same window, seed and counter.
+__device__ __forceinline__ longlong2 window_transition(long long first_tick, long long n_ticks, long long rows, unsigned long long seed,
+                                                       unsigned long long counter, long long row) {
+    const unsigned long long u = feistel_apply(feistel_make((unsigned long long)n_ticks * (unsigned long long)rows, seed, counter),
+                                               (unsigned long long)row);
+    return make_longlong2(first_tick + (long long)(u / (unsigned long long)rows), (long long)(u % (unsigned long long)rows));
+}
+
 }  // namespace tron

@@ -299,16 +299,15 @@ int launch_replay_sample_gather(const replay_ring* ring, int64_t size, int64_t k
     return cudaGetLastError() == cudaSuccess ? TRON_OK : TRON_ERR_CUDA;
 }
 
-// frame-sharing ring: transition u = (tick, row); state = frames[tick % S][row], next_state = terminal[tick % S][row] if the env
-// finished at that tick (and terminal frames are kept) else frames[(tick+1) % S][row]
+// frame-sharing ring: transition (tick, row) from window_transition (common.cuh); state = frames[tick % S][row], next_state =
+// terminal[tick % S][row] if the env finished at that tick (and terminal frames are kept) else frames[(tick+1) % S][row]
 __global__ void replay_frames_sample_gather_kernel(const replay_frames fr, long long first_tick, long long n_ticks, long long k, unsigned long long seed,
                                                    unsigned long long counter, void* out_s, void* out_s2, int out_dtype, long long* out_a, float* out_r,
                                                    float* out_d, long long* out_idx) {
     const long long row = blockIdx.x;
     if (row >= k) return;
-    const unsigned long long total = (unsigned long long)n_ticks * (unsigned long long)fr.rows;
-    const unsigned long long u = feistel_apply(feistel_make(total, seed, counter), (unsigned long long)row);
-    const long long tick = first_tick + (long long)(u / (unsigned long long)fr.rows), r = (long long)(u % (unsigned long long)fr.rows);
+    const longlong2 tr = window_transition(first_tick, n_ticks, fr.rows, seed, counter, row);
+    const long long tick = tr.x, r = tr.y;
     const long long slot = tick % fr.n_slots, nslot = (tick + 1) % fr.n_slots;
     if (!TRON_DCHECK(slot >= 0 && slot < fr.n_slots && r >= 0 && r < fr.rows, DBG_RING_SLOT)) return;
     const size_t fb = (size_t)fr.frame_elems * tron_elem(fr.frame_dtype);

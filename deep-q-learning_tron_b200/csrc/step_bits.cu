@@ -439,8 +439,8 @@ int launch_bits_import(const StepParams& p, const int8_t* tiles, bool derive_hea
 }
 
 // ------------------------------------------------------------------------------------------------ state replay ring
-// replay_states_sample_gather: transition u = (tick, row) of the window, drawn by the same Feistel permutation and (tick, row)
-// mapping as replay_frames_sample_gather.  The owning thread loads the game's planes and meta from slot tick % S, re-runs that
+// replay_states_sample_gather: transition (tick, row) of the window, drawn by window_transition (common.cuh) as in
+// replay_frames_sample_gather.  The owning thread loads the game's planes and meta from slot tick % S, re-runs that
 // tick with the recorded actions, counter and game parameters (no auto-reset: the post-tick state IS the terminal frame of a
 // game that finished) and expands the pre- and post-tick states into two Tile.value tiles.  The CTA then encodes the row's
 // player view of both through the env's plane tables, straight into the out dtype.  G transitions per CTA; output row = sample.
@@ -473,9 +473,8 @@ __global__ void __launch_bounds__(kBitsThreads) replay_states_kernel(const StepP
     const long long rows = 2ll * p.N;
     if (tid < nG) {
         const long long row = row0 + tid;
-        const unsigned long long u = feistel_apply(feistel_make((unsigned long long)q.n_ticks * (unsigned long long)rows, q.seed, q.counter_s),
-                                                   (unsigned long long)row);
-        const long long tick = q.first_tick + (long long)(u / (unsigned long long)rows), r = (long long)(u % (unsigned long long)rows);
+        const longlong2 tr = window_transition(q.first_tick, q.n_ticks, rows, q.seed, q.counter_s, row);
+        const long long tick = tr.x, r = tr.y;
         const long long slot = tick % q.S, env = r >> 1;
         const int pl = (int)(r & 1);
         if (TRON_DCHECK(slot >= 0 && slot < q.S && r >= 0 && r < rows, DBG_RING_SLOT) && TRON_DCHECK(env < p.N, DBG_ENV_OWNER)) {

@@ -9,6 +9,14 @@ Three containers:
   StateRing   -- the same transitions from the env's bit-plane state: each tick stores the pre-tick state and the actions
                  (42 B per game-tick on bits10, against 3,467 B for DDQN's frame ring), and replay_states_sample_gather re-runs
                  the sampled ticks and renders s and s' in one launch, so the horizon can be thousands of ticks.
+
+All three sample through one contract (_Sampler.sample): the same argument checks, `out=` reuse, `want_indices` and output
+tuple; each ring supplies only its length and its C entry point.  FrameRing and StateRing share one loop interface:
+
+    ring = FrameRing(env, n_slots)  or  StateRing(env, n_slots)
+    obs = ring.begin()                                          # reset; the policy reads ring.obs
+    loop:  env.select_actions(q(obs), eps, out=ring.actions_slot().view(-1)); obs = ring.step().obs
+           batch = ring.sample(64)
 """
 import ctypes as C
 
@@ -19,7 +27,49 @@ from . import _lib
 from .batch_env import _CODE_OF, _TORCH_OF, _OnDevice
 
 
-class ReplayRing:
+class _Sampler:
+    """The sampling contract of the replay rings.  A ring has `lib`, `device`, `frame_shape`, `seed` and `sample_counter`,
+    supplies __len__ (the transitions it can hand out) and _sample_call() -> (C entry point, its arguments before k)."""
+
+    def _stream(self):
+        return torch.cuda.current_stream(self.device).cuda_stream
+
+    def _next_counter(self, counter):
+        """the sampler counter of this call: `counter`, or the ring's own, which then advances"""
+        if counter is None:
+            counter, self.sample_counter = self.sample_counter, self.sample_counter + 1
+        return counter
+
+    def _outputs(self, k, out_dtype, out=None):
+        """(s, a, r, s', d) for k transitions: `out` (a tuple an earlier call returned, checked) or new tensors"""
+        if out_dtype not in (torch.float32, torch.bfloat16):
+            raise ValueError("out_dtype must be float32 or bfloat16")
+        if out is not None:
+            s = out[0]
+            if s.shape[0] != k or s.dtype != out_dtype or tuple(s.shape[1:]) != self.frame_shape:
+                raise ValueError("sample: `out` does not match k / out_dtype / the frame shape")
+            return tuple(out[:5])
+        s = torch.empty((k,) + self.frame_shape, dtype=out_dtype, device=self.device)
+        return (s, torch.empty((k, 1), dtype=torch.int64, device=self.device), torch.empty((k, 1), dtype=torch.float32, device=self.device),
+                torch.empty_like(s), torch.empty((k, 1), dtype=torch.float32, device=self.device))
+
+    def sample(self, k, out_dtype=torch.float32, counter=None, want_indices=False, out=None):
+        """k distinct transitions, uniformly (random.sample, DDQN.py:191-200), sampled and gathered in ONE launch
+        -> (s [k,*frame] out_dtype, a i64 [k,1], r f32 [k,1], s', d f32 [k,1]) (+ idx i64 [k] with want_indices).
+        out: the 5-tuple a previous call returned, to write into the same tensors again (saves five allocations per batch)."""
+        counter = self._next_counter(counter)
+        if not 0 < k <= len(self):
+            raise ValueError("sample: need 0 < k <= len(ring)=%d, got %d" % (len(self), k))
+        s, a, r, s2, d = self._outputs(k, out_dtype, out)
+        idx = torch.empty(k, dtype=torch.int64, device=self.device) if want_indices else None
+        name, head = self._sample_call()
+        with _OnDevice(self.device):
+            _lib.check(getattr(self.lib, name)(*head, k, self.seed, counter, s.data_ptr(), s2.data_ptr(), _CODE_OF[out_dtype], a.data_ptr(),
+                                               r.data_ptr(), d.data_ptr(), None if idx is None else idx.data_ptr(), self._stream()), name)
+        return (s, a, r, s2, d, idx) if want_indices else (s, a, r, s2, d)
+
+
+class ReplayRing(_Sampler):
     def __init__(self, capacity, frame_shape, frame_dtype=torch.bfloat16, device="cuda", seed=0):
         _lib.require_cuda()
         self.lib = _lib.load()
@@ -46,9 +96,6 @@ class ReplayRing:
 
     def __len__(self):
         return min(self.cursor, self.capacity)
-
-    def _stream(self):
-        return torch.cuda.current_stream(self.device).cuda_stream
 
     def push(self, state, next_state, action, reward, done, done_stride=1):
         """Append n transitions.  state/next_state: [n, *frame_shape] (ring dtype), action uint8 [n], reward f32 [n],
@@ -79,8 +126,7 @@ class ReplayRing:
             off += m
 
     def sample_indices(self, k, counter=None):
-        if counter is None:
-            counter, self.sample_counter = self.sample_counter, self.sample_counter + 1
+        counter = self._next_counter(counter)
         if not 0 < k <= len(self):
             raise ValueError("sample_indices: need 0 < k <= len(ring)=%d, got %d" % (len(self), k))
         idx = torch.empty(k, dtype=torch.int64, device=self.device)
@@ -93,49 +139,22 @@ class ReplayRing:
         """-> (states [k,*frame], actions i64 [k,1], rewards f32 [k,1], next_states, dones f32 [k,1])  (DDQN.py:191-200)"""
         idx = idx.to(device=self.device, dtype=torch.int64).contiguous()
         k = idx.numel()
-        if out_dtype not in (torch.float32, torch.bfloat16):
-            raise ValueError("gather: out_dtype must be float32 or bfloat16")
-        s = torch.empty((k,) + self.frame_shape, dtype=out_dtype, device=self.device)
-        s2 = torch.empty_like(s)
-        a = torch.empty((k, 1), dtype=torch.int64, device=self.device)
-        r = torch.empty((k, 1), dtype=torch.float32, device=self.device)
-        d = torch.empty((k, 1), dtype=torch.float32, device=self.device)
+        s, a, r, s2, d = self._outputs(k, out_dtype)
         with _OnDevice(self.device):
             _lib.check(self.lib.replay_gather(C.byref(self.ring), idx.data_ptr(), k, s.data_ptr(), s2.data_ptr(), _CODE_OF[out_dtype],
                                               a.data_ptr(), r.data_ptr(), d.data_ptr(), self._stream()), "replay_gather")
         return s, a, r, s2, d
 
-    def _outputs(self, k, out_dtype):
-        if out_dtype not in (torch.float32, torch.bfloat16):
-            raise ValueError("out_dtype must be float32 or bfloat16")
-        s = torch.empty((k,) + self.frame_shape, dtype=out_dtype, device=self.device)
-        return (s, torch.empty((k, 1), dtype=torch.int64, device=self.device), torch.empty((k, 1), dtype=torch.float32, device=self.device),
-                torch.empty_like(s), torch.empty((k, 1), dtype=torch.float32, device=self.device))
-
-    def sample(self, k, out_dtype=torch.float32, counter=None, want_indices=False, out=None):
-        """k distinct transitions, uniformly (random.sample, DDQN.py:191-200), sampled and gathered in ONE launch.
-        out: the 5-tuple a previous call returned, to write into the same tensors again (saves five allocations per batch)."""
-        if counter is None:
-            counter, self.sample_counter = self.sample_counter, self.sample_counter + 1
-        if not 0 < k <= len(self):
-            raise ValueError("sample: need 0 < k <= len(ring)=%d, got %d" % (len(self), k))
-        s, a, r, s2, d = out[:5] if out is not None else self._outputs(k, out_dtype)
-        if out is not None and (s.shape[0] != k or s.dtype != out_dtype or tuple(s.shape[1:]) != self.frame_shape):
-            raise ValueError("sample: `out` does not match k / out_dtype / the frame shape")
-        idx = torch.empty(k, dtype=torch.int64, device=self.device) if want_indices else None
-        with _OnDevice(self.device):
-            _lib.check(self.lib.replay_sample_gather(C.byref(self.ring), len(self), k, self.seed, counter, s.data_ptr(), s2.data_ptr(),
-                                                     _CODE_OF[out_dtype], a.data_ptr(), r.data_ptr(), d.data_ptr(),
-                                                     None if idx is None else idx.data_ptr(), self._stream()), "replay_sample_gather")
-        return (s, a, r, s2, d, idx) if want_indices else (s, a, r, s2, d)
+    def _sample_call(self):
+        return "replay_sample_gather", (C.byref(self.ring), len(self))
 
 
-class FrameRing:
+class FrameRing(_Sampler):
     """Frame-sharing replay ring for a BatchedTron: S time slots of [rows = 2N] frames.
 
         ring = FrameRing(env, n_slots)
-        obs = ring.begin(env)                                  # reset observation lands in slot 0
-        loop:  act = policy(ring.frames(t)); ring.step(env, act)   # tick t -> obs of tick t+1 lands in slot (t+1) % S
+        obs = ring.begin()                                     # reset observation lands in slot 0
+        loop:  act = policy(ring.obs); ring.step(act)          # tick t -> obs of tick t+1 lands in slot (t+1) % S
                batch = ring.sample(64)
 
     Transition (t, row): state = slot t % S, action/reward/done stored in slot t % S, next_state = slot (t+1) % S, or the
@@ -161,32 +180,40 @@ class FrameRing:
         self.reward_t = torch.zeros((self.S, N, 2), dtype=torch.float32, device=self.device)
         self.done_t = torch.zeros((self.S, N), dtype=torch.uint8, device=self.device)
         self.winner = torch.empty(N, dtype=torch.uint8, device=self.device)
-        self.tick = 0  # ticks played: transitions of ticks [max(0, tick - (S-1)), tick) are complete
+        self.tick = 0  # ticks played
         self.seed, self.sample_counter = int(seed), 0
         self.fr = abi.ReplayFrames(struct_size=C.sizeof(abi.ReplayFrames), frame_elems=self.F, frame_dtype=self.dt, n_slots=self.S, rows=self.rows,
                                    frames=self.frames_t.data_ptr(), terminal=None if self.terminal_t is None else self.terminal_t.data_ptr(),
                                    action=self.action_t.data_ptr(), reward=self.reward_t.data_ptr(), done=self.done_t.data_ptr())
 
+    def _window(self):
+        """(first_tick, n_ticks): the ticks whose transitions are complete, the last min(tick, S-1) (slot t+1 holds s' of tick t)"""
+        n = min(self.tick, self.S - 1)
+        return self.tick - n, n
+
     def __len__(self):
-        return min(self.tick, self.S - 1) * self.rows
+        return self._window()[1] * self.rows
 
     def frames(self, tick=None):
         """the observation the policy sees at `tick` (default: the current one): [N, 2, P, W+2, H+2], a view of the ring"""
         return self.frames_t[(self.tick if tick is None else tick) % self.S]
 
-    def begin(self, env=None, spawn=None):
-        env = env or self.env
+    @property
+    def obs(self):
+        """the observation the policy reads now: frames()"""
+        return self.frames()
+
+    def begin(self, spawn=None):
         self.tick = 0
-        return env.reset(spawn=spawn, obs=self.frames_t[0])
+        return self.env.reset(spawn=spawn, obs=self.frames_t[0])
 
     def actions_slot(self):
         """uint8 [N,2] view the policy writes the actions of the current tick into (select_actions(out=...))"""
         return self.action_t[self.tick % self.S]
 
-    def step(self, env=None, actions=None, **kw):
+    def step(self, actions=None, **kw):
         """one env tick whose outputs land in the ring; actions None -> the ones already written into actions_slot()"""
-        env = env or self.env
-        t, S = self.tick, self.S
+        env, t, S = self.env, self.tick, self.S
         slot, nslot = t % S, (t + 1) % S
         if actions is not None:
             self.action_t[slot].copy_(actions.reshape(env.N, 2))
@@ -195,36 +222,11 @@ class FrameRing:
         self.tick = t + 1
         return res
 
-    def sample(self, k, out_dtype=torch.float32, counter=None, want_indices=False, out=None):
-        """k distinct complete transitions, uniformly, one launch -> (s, a i64 [k,1], r f32 [k,1], s', d f32 [k,1]).
-        out: the 5-tuple a previous call returned, to write into the same tensors again (saves five allocations per batch)."""
-        n_ticks = min(self.tick, self.S - 1)
-        if counter is None:
-            counter, self.sample_counter = self.sample_counter, self.sample_counter + 1
-        if not 0 < k <= n_ticks * self.rows:
-            raise ValueError("sample: need 0 < k <= %d complete transitions, got %d" % (n_ticks * self.rows, k))
-        if out_dtype not in (torch.float32, torch.bfloat16):
-            raise ValueError("out_dtype must be float32 or bfloat16")
-        if out is not None:
-            s, a, r, s2, d = out[:5]
-            if s.shape[0] != k or s.dtype != out_dtype or tuple(s.shape[1:]) != self.frame_shape:
-                raise ValueError("sample: `out` does not match k / out_dtype / the frame shape")
-        else:
-            s = torch.empty((k,) + self.frame_shape, dtype=out_dtype, device=self.device)
-            s2 = torch.empty_like(s)
-            a = torch.empty((k, 1), dtype=torch.int64, device=self.device)
-            r = torch.empty((k, 1), dtype=torch.float32, device=self.device)
-            d = torch.empty((k, 1), dtype=torch.float32, device=self.device)
-        idx = torch.empty(k, dtype=torch.int64, device=self.device) if want_indices else None
-        with _OnDevice(self.device):
-            _lib.check(self.lib.replay_frames_sample_gather(C.byref(self.fr), self.tick - n_ticks, n_ticks, k, self.seed, counter, s.data_ptr(),
-                                                            s2.data_ptr(), _CODE_OF[out_dtype], a.data_ptr(), r.data_ptr(), d.data_ptr(),
-                                                            None if idx is None else idx.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream),
-                       "replay_frames_sample_gather")
-        return (s, a, r, s2, d, idx) if want_indices else (s, a, r, s2, d)
+    def _sample_call(self):
+        return "replay_frames_sample_gather", (C.byref(self.fr),) + self._window()
 
 
-class StateRing:
+class StateRing(_Sampler):
     """Replay ring of env states for a BatchedTron on a bit-plane layout: S time slots, each the state blob (planes + meta) BEFORE
     tick t, the actions of tick t and the RNG counter it ran with (plus the temper mode's game parameters).  A transition
     (s, a, r, s', d) is re-simulated when it is sampled: the sample kernel re-runs tick t of the game with tron_step's rules and
@@ -232,12 +234,13 @@ class StateRing:
     frames.  Drop-in for FrameRing in a training loop:
 
         ring = StateRing(env, n_slots)
-        obs = ring.begin(obs=buf)                                   # the policy reads `buf`, refreshed in place every tick
-        loop:  env.select_actions(q, eps, counter=env.counter, out=ring.actions_slot().view(-1)); ring.step(obs=buf)
+        obs = ring.begin()                                          # the policy reads ring.obs, refreshed in place every tick
+        loop:  env.select_actions(q, eps, counter=env.counter, out=ring.actions_slot().view(-1)); obs = ring.step().obs
                batch = ring.sample(64)
 
-    Same (seed, counter) and window as a FrameRing -> the same sampled transitions, bit for bit.  Passing one reused `obs` buffer
-    lets BatchedTron.step store only the parts of each row that a tick changes.
+    Same (seed, counter) and window as a FrameRing -> the same sampled transitions, bit for bit.  `obs` is one buffer that every
+    step reuses, which lets BatchedTron.step store only the parts of each row that a tick changes; begin(obs=buf) or
+    step(obs=buf) makes `buf` that buffer.
     """
 
     def __init__(self, env, n_slots, seed=0):
@@ -264,27 +267,36 @@ class StateRing:
         self.action_t = torch.zeros((self.S, N, 2), dtype=torch.uint8, device=self.device)
         self.counter_t = torch.zeros(self.S, dtype=torch.int64, device=self.device)
         self.params_t = torch.zeros((self.S, N, 4), dtype=torch.int8, device=self.device) if env.slide_mode == abi.SLIDE_TEMPER else None
-        self.tick = 0  # ticks played: transitions of ticks [max(0, tick - S), tick) are in the ring
+        self.obs = env.new_obs()  # the observation the policy reads now
+        self.tick = 0  # ticks played
         self.seed, self.sample_counter = int(seed), 0
         self.rs = abi.ReplayStates(struct_size=C.sizeof(abi.ReplayStates), n_slots=self.S, slot_bytes=slot_bytes, states=self.states_t.data_ptr(),
                                    action=self.action_t.data_ptr(), counter=self.counter_t.data_ptr(),
                                    slide_params=None if self.params_t is None else self.params_t.data_ptr())
 
+    def _window(self):
+        """(first_tick, n_ticks): the ticks in the ring, the last min(tick, S) (s' is re-simulated, no slot holds it)"""
+        n = min(self.tick, self.S)
+        return self.tick - n, n
+
     def __len__(self):
-        return min(self.tick, self.S) * self.rows
+        return self._window()[1] * self.rows
 
     def begin(self, spawn=None, obs=None):
-        """reset the env (its first observation lands in `obs`, default a new buffer) and start at tick 0"""
+        """reset the env (its first observation lands in `obs`, which becomes self.obs) and start at tick 0"""
+        if obs is not None:
+            self.obs = obs
         self.tick = 0
-        return self.env.reset(spawn=spawn, obs=obs)
+        return self.env.reset(spawn=spawn, obs=self.obs)
 
     def actions_slot(self):
         """uint8 [N,2] view the policy writes the actions of the current tick into (select_actions(out=...))"""
         return self.action_t[self.tick % self.S]
 
     def step(self, actions=None, obs=None, **kw):
-        """record the pre-tick state, then one env tick; actions None -> the ones already written into actions_slot().
-        All on the env's stream, so the step can be captured in a CUDA graph (with env.use_device_counter())."""
+        """record the pre-tick state, then one env tick into self.obs (or `obs`, which becomes self.obs); actions None -> the ones
+        already written into actions_slot().  All on the env's stream, so the step can be captured in a CUDA graph (with
+        env.use_device_counter())."""
         env, slot = self.env, self.tick % self.S
         if actions is not None:
             self.action_t[slot].copy_(actions.reshape(env.N, 2))
@@ -297,35 +309,11 @@ class StateRing:
             self.counter_t[slot].fill_(env.counter)
         if self.params_t is not None:
             self.params_t[slot].copy_(env.slide_params)
-        res = env.step(self.action_t[slot], obs=obs, want_ep_len=False, **kw)
+        if obs is not None:
+            self.obs = obs
+        res = env.step(self.action_t[slot], obs=self.obs, want_ep_len=False, **kw)
         self.tick += 1
         return res
 
-    def sample(self, k, out_dtype=torch.float32, counter=None, want_indices=False, out=None):
-        """k distinct transitions of the last min(tick, S) ticks, uniformly, one launch -> (s, a i64 [k,1], r f32 [k,1], s', d f32 [k,1]),
-        as FrameRing.sample.  out: the 5-tuple a previous call returned, to write into the same tensors again."""
-        n_ticks = min(self.tick, self.S)
-        if counter is None:
-            counter, self.sample_counter = self.sample_counter, self.sample_counter + 1
-        if not 0 < k <= n_ticks * self.rows:
-            raise ValueError("sample: need 0 < k <= %d transitions, got %d" % (n_ticks * self.rows, k))
-        if out_dtype not in (torch.float32, torch.bfloat16):
-            raise ValueError("out_dtype must be float32 or bfloat16")
-        if out is not None:
-            s, a, r, s2, d = out[:5]
-            if s.shape[0] != k or s.dtype != out_dtype or tuple(s.shape[1:]) != self.frame_shape:
-                raise ValueError("sample: `out` does not match k / out_dtype / the frame shape")
-        else:
-            s = torch.empty((k,) + self.frame_shape, dtype=out_dtype, device=self.device)
-            s2 = torch.empty_like(s)
-            a = torch.empty((k, 1), dtype=torch.int64, device=self.device)
-            r = torch.empty((k, 1), dtype=torch.float32, device=self.device)
-            d = torch.empty((k, 1), dtype=torch.float32, device=self.device)
-        idx = torch.empty(k, dtype=torch.int64, device=self.device) if want_indices else None
-        args = self.env._args()
-        with _OnDevice(self.device):
-            _lib.check(self.lib.replay_states_sample_gather(C.byref(self.rs), C.byref(args), self.tick - n_ticks, n_ticks, k, self.seed, counter,
-                                                            s.data_ptr(), s2.data_ptr(), _CODE_OF[out_dtype], a.data_ptr(), r.data_ptr(), d.data_ptr(),
-                                                            None if idx is None else idx.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream),
-                       "replay_states_sample_gather")
-        return (s, a, r, s2, d, idx) if want_indices else (s, a, r, s2, d)
+    def _sample_call(self):
+        return "replay_states_sample_gather", (C.byref(self.rs), C.byref(self.env._args())) + self._window()

@@ -1,7 +1,7 @@
 """The state replay ring (StateRing, replay_states_sample_gather): it stores each tick's pre-tick env state and actions and
 re-simulates sampled transitions.  Checked bit for bit against the frame ring driven by a twin env, against explicit transitions
-(oracle and GPU), over a long horizon, under a captured CUDA graph with the device counter, in the debug build and in the
-training loops."""
+(oracle and GPU), over a long horizon, under a captured CUDA graph with the device counter, on its own reused obs buffer, in the
+debug build and in the training loops; plus the status codes of every sample / gather entry point."""
 import ctypes as C
 import os
 import subprocess
@@ -231,6 +231,32 @@ def test_state_ring_device_counter_graph():
             assert np.array_equal(_bits(w), _bits(g))
 
 
+@pytest.mark.gpu
+def test_state_ring_steps_its_own_obs_buffer():
+    """a StateRing begun without a buffer steps its own `obs`: one tensor every tick, which the env reports as holding the previous
+    observation (so BatchedTron.step stores only the changed parts of each row); its samples equal a twin ring's on an explicit
+    buffer"""
+    from tron_b200.replay import StateRing
+    N, S, T = 300, 4, 11
+    ea, eb = _env(N, 10, 10, "bits10", abi.BF16, "popup3"), _env(N, 10, 10, "bits10", abi.BF16, "popup3")
+    sr, twin = StateRing(ea, S, seed=9), StateRing(eb, S, seed=9)
+    assert sr.begin() is sr.obs
+    ptr = sr.obs.data_ptr()
+    tobs = twin.begin(obs=eb.new_obs())
+    rng = np.random.default_rng(2)
+    for t in range(T):
+        a = _tape(rng, N)
+        assert ea._obs_is_prev(sr.obs), t
+        res = sr.step(actions=a)
+        assert res.obs is sr.obs and sr.obs.data_ptr() == ptr, t
+        twin.step(actions=a, obs=tobs)
+        assert np.array_equal(_bits(sr.obs), _bits(tobs)), t
+        for k in (64, len(sr)):
+            for name, w, g in zip(("s", "a", "r", "s2", "d", "idx"), twin.sample(k, counter=t, want_indices=True),
+                                  sr.sample(k, counter=t, want_indices=True)):
+                assert np.array_equal(_bits(w), _bits(g)), (t, k, name)
+
+
 def _call(sr, env_args, first, n_ticks, k, out, out_dtype=abi.F32, rs=None):
     from tron_b200 import _lib
     s, a, r, s2, d = out
@@ -288,6 +314,50 @@ def test_state_ring_refusals():
         assert _call(sr, a2, 0, 2, 64, good) == abi.ERR_UNSUPPORTED, layout
     with pytest.raises(_lib.TronError):
         _lib.check(_call(sr, args, 0, S + 1, 64, good), "replay_states_sample_gather")
+
+
+@pytest.mark.gpu
+def test_sample_gather_status_codes():
+    """replay_gather, replay_sample_gather and replay_frames_sample_gather on real, correctly sized buffers: the valid call returns
+    OK and every refused call differs from it in exactly one argument"""
+    from tron_b200 import _lib
+    from tron_b200.batch_env import BatchedTron
+    from tron_b200.replay import FrameRing, ReplayRing
+    lib, stream = _lib.load(), torch.cuda.current_stream().cuda_stream
+    k, F = 64, 3 * 144
+    buf = torch.zeros(2 * k * F + 16, dtype=torch.float32, device="cuda")
+    side = [torch.zeros((k, 1), dtype=dt, device="cuda") for dt in (torch.int64, torch.float32, torch.float32)]
+    good = [buf.data_ptr(), buf.data_ptr() + k * F * 4] + [t.data_ptr() for t in side]  # s, s', a, r, d
+    idx = torch.arange(k, dtype=torch.int64, device="cuda")
+    ring = ReplayRing(256, (3, 12, 12), torch.bfloat16)
+    fr = FrameRing(BatchedTron(k, 10, 10, layout="bits10", obs_dtype=torch.bfloat16, obs_enc="popup3"), 3, keep_terminal=True)
+
+    def gather(rg, win, o, dt):
+        return lib.replay_gather(C.byref(rg), idx.data_ptr(), k, o[0], o[1], dt, o[2], o[3], o[4], stream)
+
+    def sample_gather(rg, win, o, dt):  # win = size
+        return lib.replay_sample_gather(C.byref(rg), win, k, 0, 0, o[0], o[1], dt, o[2], o[3], o[4], None, stream)
+
+    def frames_sample_gather(rg, win, o, dt):  # win = (first_tick, n_ticks)
+        return lib.replay_frames_sample_gather(C.byref(rg), win[0], win[1], k, 0, 0, o[0], o[1], dt, o[2], o[3], o[4], None, stream)
+
+    for call, rg, ring_ptrs, win, past in ((gather, ring.ring, ("state", "next_state"), None, []),
+                                           (sample_gather, ring.ring, ("state", "next_state"), 256, [257, k - 1]),
+                                           (frames_sample_gather, fr.fr, ("frames", "terminal"), (0, 2), [(0, 3), (-1, 2)])):
+        name = call.__name__
+        assert call(rg, win, good, abi.F32) == abi.OK, name
+        torch.cuda.synchronize()
+        for i in range(5):
+            assert call(rg, win, good[:i] + [None] + good[i + 1:], abi.F32) == abi.ERR_INVALID, (name, i)
+        assert call(rg, win, good, abi.I8) == abi.ERR_INVALID, name
+        assert call(rg, win, [good[0] + 4] + good[1:], abi.F32) == abi.ERR_ALIGN, name
+        assert call(rg, win, good[:1] + [good[1] + 8] + good[2:], abi.F32) == abi.ERR_ALIGN, name
+        for field in ring_ptrs:
+            bad = type(rg).from_buffer_copy(rg)
+            setattr(bad, field, getattr(rg, field) + 4)
+            assert call(bad, win, good, abi.F32) == abi.ERR_ALIGN, (name, field)
+        for w in past:  # a window past the ring: size > capacity or k > size; n_ticks > S - 1 or first_tick < 0
+            assert call(rg, w, good, abi.F32) == abi.ERR_INVALID, (name, w)
 
 
 @pytest.mark.gpu

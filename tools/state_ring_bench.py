@@ -45,13 +45,13 @@ def rings(N, dt, enc, window):
     eb = BatchedTron(N, 10, 10, obs_dtype=dt, obs_enc=enc, seed=0, layout="bits10")
     fr, sr = FrameRing(ea, window + 1, keep_terminal=True, seed=1), StateRing(eb, window, seed=1)
     fr.begin()
-    obs = sr.begin(obs=eb.new_obs())
+    sr.begin()
     for _ in range(window):
         a = ea.random_actions()
         fr.step(actions=a)
-        sr.step(actions=a, obs=obs)
+        sr.step(actions=a)
     torch.cuda.synchronize()
-    return fr, sr, obs
+    return fr, sr
 
 
 def main():
@@ -73,7 +73,7 @@ def main():
 
     # ---- one sample launch, k = 64 / 1024 / 4096, 65,536 games, an 8-tick window
     for name, (dt, enc, odt) in CASES.items():
-        fr, sr, _ = rings(args.sample_games, dt, enc, 8)
+        fr, sr = rings(args.sample_games, dt, enc, 8)
         for k in (64, 1024, 4096):
             us = {}
             for label, ring in (("frames", fr), ("states", sr)):
@@ -87,15 +87,15 @@ def main():
     # ---- one step() of each ring and bytes per game-tick (DDQN configuration)
     dt, enc, _ = CASES["ddqn_bf16_popup3_to_f32"]
     for N in args.step_games:
-        fr, sr, obs = rings(N, dt, enc, 2)
+        fr, sr = rings(N, dt, enc, 2)
         f_us = device_us(lambda: fr.step(), calls=10, replays=10)
-        s_us = device_us(lambda: sr.step(obs=obs), calls=10, replays=10)
+        s_us = device_us(lambda: sr.step(), calls=10, replays=10)
         emit(what="step_device_us", case="ddqn_bf16_popup3", games=N, frames_us=round(f_us, 2), states_us=round(s_us, 2),
              frames_bytes_per_game_tick=round(ring_bytes(fr) / (fr.S * N), 2), states_bytes_per_game_tick=round(ring_bytes(sr) / (sr.S * N), 2))
-        del fr, sr, obs
+        del fr, sr
         torch.cuda.empty_cache()
     for name, (dt, enc, _) in CASES.items():
-        fr, sr, _ = rings(4096, dt, enc, 2)
+        fr, sr = rings(4096, dt, enc, 2)
         emit(what="bytes_per_game_tick", case=name, frames=round(ring_bytes(fr) / (fr.S * 4096), 2), states=round(ring_bytes(sr) / (sr.S * 4096), 2))
 
     # ---- the DDQN loop: env_replay_ms per tick (select_actions + ring step), frames vs states
