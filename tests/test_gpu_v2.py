@@ -338,10 +338,14 @@ def test_bound_step_equals_step():
 
 def test_tuning_options_do_not_change_results():
     """CTA caps (shared-memory padding) and the store-schedule switch are performance knobs only: identical outputs"""
+    import _geometry as geo
     from tron_b200 import _lib
     from tron_b200.batch_env import BatchedTron
     L = _lib.load()
-    N = 1 << 17  # more than 8 CTAs per SM, so the caps are active
+    sms = geo.sm_count()
+    N = 1 << 18  # 128 games per CTA and 2,048 CTAs on 148 SMs: more than 8 CTAs per SM, so the caps pad shared memory
+    codes = {torch.bfloat16: abi.BF16, torch.float32: abi.F32, torch.int8: abi.I8}
+    encs = {"lut1": abi.ENC_LUT1, "popup3": abi.ENC_POPUP3}
 
     def run(layout, enc, dtype, slide=None):
         env = BatchedTron(N, 10, 10, obs_dtype=dtype, obs_enc=enc, seed=12, layout=layout, slide_mode=slide)
@@ -349,10 +353,24 @@ def test_tuning_options_do_not_change_results():
         for _ in range(3):
             r = env.step()
         return r.obs.clone().view(torch.uint8), r.reward.clone(), env.export()["tiles"].clone()
+
+    def want_geometry(layout, enc, dtype, slide, opt):
+        if layout == "tile8":
+            return geo.tile_geometry(N, 10, 10, codes[dtype], encs[enc], sms, cap_opt=opt[1] if opt[0] == abi.OPT_TILE_CTAS_PER_SM else 0)
+        return geo.bits_geometry(N, 10, 10, layout, codes[dtype], encs[enc], False, sms, cap_opt=opt[1] if opt[0] == abi.OPT_BITS_CTAS_PER_SM else 0)
     cases = [("bits10", "lut1", torch.bfloat16, None), ("bits10", "popup3", torch.int8, None), ("bits", "lut1", torch.float32, "temper"), ("tile8", "popup3", torch.bfloat16, None)]
+    opts = ((abi.OPT_BITS_CTAS_PER_SM, 2), (abi.OPT_BITS_CTAS_PER_SM, 32), (abi.OPT_TILE_CTAS_PER_SM, 3), (abi.OPT_ENCODE_VARIANT, 8))
+    # the geometry guard: every case under every setting launches with 128 games per CTA, 2,048 CTAs and the padding its cap gives
+    probes = [(c, o) for o in [(0, 0)] + list(opts) for c in cases]
+    launched = geo.step_launches_in_fresh_process([dict(env=dict(n_envs=N, width=10, height=10, obs_dtype=str(c[2]).split(".")[1], obs_enc=c[1], seed=12,
+                                                                 layout=c[0], slide_mode=c[3]), options=[o] if o[0] else []) for c, o in probes])
+    for (c, o), got in zip(probes, launched):
+        want = want_geometry(*c, o)
+        assert want.G == 128 and want.grid > 8 * sms
+        geo.assert_geometry(got, want, (c, o))
     try:
         base = [run(*c) for c in cases]
-        for opt, val in ((abi.OPT_BITS_CTAS_PER_SM, 2), (abi.OPT_BITS_CTAS_PER_SM, 32), (abi.OPT_TILE_CTAS_PER_SM, 3), (abi.OPT_ENCODE_VARIANT, 8)):
+        for opt, val in opts:
             _lib.check(L.tron_set_option(opt, val))
             for c, want in zip(cases, base):
                 got = run(*c)
