@@ -248,8 +248,8 @@ __global__ void __launch_bounds__(kBitsThreads) step_bits_kernel(const StepParam
     const long long env = env0 + tid;
     Cells g;
     g.clear(); g.Wr = p.W; g.Hr = p.H;
-    EnvState e = unpack_meta(make_uint2(0, 0));
-    if (owner) {
+    EnvState e = unpack_meta(make_uint2(0, 0)); int pre[2] = {0, 0};  // delta: the tick's actions, issued before the planes and meta
+    if (owner) { if (delta && p.actions) for (int i = 0; i < 2; ++i) pre[i] = read_action(p.actions, p.action_dtype, 2 * (size_t)env + i);
         if (!(MODE == MODE_RESET && p.env_mask == nullptr)) set_planes(g, load_planes<SLIDE>(p, env));
         e = unpack_meta(p.meta[env]);
     }
@@ -261,7 +261,7 @@ __global__ void __launch_bounds__(kBitsThreads) step_bits_kernel(const StepParam
         const int hp1 = delta ? head_cell10(e.r1, e.c1) : 0, hp2 = delta ? head_cell10(e.r2, e.c2) : 0;
         if (MODE != MODE_OBSERVE && owner) {
             BoxRegs bx;
-            fin = env_tick<MODE, false, (SLIDE ? FEAT_ALL : FEAT_EPS)>(g, p, e, env, t, tid, bx);  // BITS10 has no slide plane
+            fin = env_tick<MODE, false, (SLIDE ? FEAT_ALL : FEAT_EPS)>(g, p, e, env, t, tid, bx, (delta && p.actions) ? pre : nullptr);  // BITS10: no slide plane
         }
         if constexpr (LP > 0 && MODE == MODE_STEP) {
             if (p.obs_term) {  // last frame of the games that just finished (-> obs_terminal)
